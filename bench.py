@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric on BASELINE.json's config, one JSON line on stdout (rank 0).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Workload (config.workload): BASELINE configs[1] -- 1080p60 geometry (1125 total lines, the GUI's convention;
@@ -18,6 +18,10 @@ One STEP = 80 batches (~57 ms of device time), so that the default 20 steps time
           the way the reference arm is measured.  `e2e.pinned_process` beside it: tsdrgpu_pipeline_process_raw_async() on
           page-locked host IQ (a front end that owns page-locked buffers), `e2e_int8_transport`: the same with 8-bit samples.
 N > 1     N independent streams, one per GPU (the path has no cross-stream exchange: replicas, weak scaling).
+--dump-outputs DIR  after the timed steps, rank 0 writes what the last of them handed out, so that two builds can be compared
+          output for output (the inputs are seeded): DIR/frames.npy, the last frames of the last batch (float32, at most
+          48 MB of them, one row per frame), and DIR/frame_plot.npy, DIR/line_plot.npy, the frame-rate detector's two lag
+          plots (float64).
 --impl reference   the reference's own threaded CPU pipeline (oracle/_ref: libTSDRLibrary.so + its RawFile plugin
           with pacing off) on this box's host cores, same geometry; falls back to the pinned C port when the
           reference binary is absent.
@@ -149,6 +153,7 @@ class DeviceStep:
         self.mag = self.mags[0]
         self.mag_fill = 0
         self.frames = 0
+        self.last_frames = 0                                # frames the last batch wrote to frames_out[(k - 1) & 1]
         self.captures = 0
         self.k = 0
         self.chunk = int(os.environ.get("BENCH_FRAME_CHUNK", "0"))
@@ -185,6 +190,7 @@ class DeviceStep:
             done += nf
         self.k += 1
         self.frames += done
+        self.last_frames = done
         # frame-rate detector: the whole stream is demodulated once; every complete capture of 3.1*fs/55 samples is
         # autocorrelated (batched FFTs) and accumulated in order
         if not fused_mag:
@@ -213,6 +219,16 @@ class DeviceStep:
     def join(self):
         self.pp.join()
         self.frd.join()
+
+    def dump_outputs(self, path):
+        """The frames of the last batch (the last ones, at most 48 MB) and the detector's lag plots as .npy files; call after join()."""
+        os.makedirs(path, exist_ok=True)
+        keep = max(1, min(self.last_frames, (48 << 20) // (4 * self.n)))
+        frames = self.frames_out[(self.k - 1) & 1][(self.last_frames - keep) * self.n: self.last_frames * self.n]
+        np.save(os.path.join(path, "frames.npy"), frames.view(keep, self.n).cpu().numpy())
+        (_, frame_plot), (_, line_plot) = self.frd.plots(FS)
+        np.save(os.path.join(path, "frame_plot.npy"), frame_plot)
+        np.save(os.path.join(path, "line_plot.npy"), line_plot)
 
 
 def collect_profile(gpu):
@@ -449,6 +465,8 @@ def run_ours(args):
     launches = gpu.launches - launches0
     frames_done, caps_done = batch.frames - frames0, batch.captures - caps0
     value = world * args.steps * pairs_step / (ms_total * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        batch.dump_outputs(args.dump_outputs)
 
     if os.environ.get("BENCH_QUICK"):                 # used under ncu and for the opt-in variants: the timed steps only
         if rank == 0:
@@ -1089,6 +1107,7 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "reference_child"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR as .npy files")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -1,7 +1,14 @@
 """Golden vectors captured from the REAL reference (tests/golden/make_golden.py) checked against
   * the C restatement  (CPU, always), and
   * the CUDA path      (tests/test_gpu_parity.py reuses `load` from here on the GPU box).
+
+The scenario tests that compare with the reference (test_oracle_pinning, test_host_library, test_rawfile_plugin) read what
+the reference returned from tests/golden/reference_outputs.json (tests/golden/make_reference_outputs.py): scalars as they
+are, arrays as a digest of their bits (`observed`), so that a bit-exact comparison needs no stored array.
 """
+import hashlib
+import json
+import math
 import os
 
 import numpy as np
@@ -11,10 +18,44 @@ from oracle import oracle as orc
 from tempestsdr_b200 import synth
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+REFERENCE_OUTPUTS = os.path.join(GOLD, "reference_outputs.json")
 
 
 def load(name):
     return np.load(os.path.join(GOLD, name))
+
+
+def observed(v):
+    """A JSON-comparable form of what a scenario observed: arrays become dtype, shape and a SHA-256 of their bits (equal
+    digests mean bit-identical arrays), tuples become lists, bytes become text, NaN becomes the string "nan"."""
+    if isinstance(v, np.ndarray):
+        a = np.ascontiguousarray(v)
+        return f"{a.dtype.str}{list(a.shape)}:{hashlib.sha256(a.tobytes()).hexdigest()[:32]}"
+    if isinstance(v, (list, tuple)):
+        return [observed(x) for x in v]
+    if isinstance(v, bytes):
+        return v.decode("latin-1")
+    if isinstance(v, np.generic):
+        v = v.item()
+    if isinstance(v, float) and math.isnan(v):
+        return "nan"
+    return v
+
+
+def reference_outputs(key):
+    """What the compiled reference returned in scenario `key`, as recorded by make_reference_outputs.py."""
+    with open(REFERENCE_OUTPUTS) as f:
+        return json.load(f)[key]
+
+
+def assert_matches_reference(key, observations):
+    """`observations`: (label, value) pairs from one scenario run against this project's code; compared one by one with the
+    reference's values for the same scenario."""
+    want = reference_outputs(key)
+    got = [(label, observed(v)) for label, v in observations]
+    assert len(got) == len(want), f"{key}: {len(got)} observations, the reference made {len(want)}"
+    bad = [(label, g, w) for (label, g), w in zip(got, want) if g != w]
+    assert not bad, f"{key}: {len(bad)} of {len(got)} differ from the reference, first: {bad[0]}"
 
 
 def same_bits(a, b):

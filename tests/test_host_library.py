@@ -1,10 +1,14 @@
 """The C host library (tempestsdr_b200/lib/libTSDRLibrary.so): same exported tsdr_* symbols, status codes and
-error-text behaviour as the reference library, exercised with the REFERENCE's own unmodified RawFile source plugin
-(oracle/_ref/libTSDRPlugin_RawFile*.so -- a source plugin under test, not an oracle).  CPU part here; the GPU
-end-to-end run is test_host_library_end_to_end (marked gpu)."""
+error-text behaviour as the reference library.  The reference's side of each comparison is what the compiled reference
+library did in the same scenario with the reference's own RawFile source plugin, recorded in
+tests/golden/reference_outputs.json; this library runs it with this project's RawFile plugin in its plain ten-symbol
+mode (test_rawfile_plugin pins that plugin to the reference's).  CPU part here; the GPU end-to-end run is
+test_host_library_end_to_end (marked gpu)."""
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 import threading
 import time
 
@@ -13,9 +17,11 @@ import pytest
 
 from oracle import oracle as orc
 from tempestsdr_b200 import synth
+from tests.test_golden import assert_matches_reference, reference_outputs
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 MINE = os.path.join(ROOT, "tempestsdr_b200", "lib", "libTSDRLibrary.so")
+PLUGIN = os.path.join(ROOT, "tempestsdr_b200", "lib", "TSDRPlugin_RawFileGPU.so")
 
 FRAME_CB = C.CFUNCTYPE(None, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_void_p)
 VALUE_CB = C.CFUNCTYPE(None, C.c_int, C.c_double, C.c_double, C.c_void_p)
@@ -47,101 +53,116 @@ def exported(path, prefix):
     return sorted(l.split()[-1] for l in out.splitlines() if l.split()[-1].startswith(prefix))
 
 
-needs_ref = pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built")
+def plugin_error_text(plugin, params, tmp_path):
+    """The text `plugin` itself reports when its init rejects `params`: run on a private copy of it, so that the copy the
+    library loads keeps its own state (a plugin keeps its state in statics)."""
+    copy = os.path.join(tempfile.mkdtemp(dir=tmp_path), os.path.basename(plugin))     # a fresh file: a loaded one is never overwritten
+    shutil.copy(plugin, copy)
+    lib = C.CDLL(copy)
+    lib.tsdrplugin_getlasterrortext.restype = C.c_char_p
+    assert lib.tsdrplugin_init(C.create_string_buffer(params.encode())) != 0      # a plugin may tokenise its parameters in place
+    return lib.tsdrplugin_getlasterrortext()
 
 
-@needs_ref
+def forwarded(text, plugin_text):
+    """A library hands a plugin's rejection text on to the host: that text is the plugin's own, so what is compared is that
+    it was forwarded unchanged."""
+    return "<the plugin's own error text>" if text == plugin_text else text
+
+
 def test_same_exported_api_as_the_reference_library():
-    assert exported(MINE, "tsdr_") == exported(orc.REF_LIB_SO, "tsdr_")
+    assert exported(MINE, "tsdr_") == reference_outputs("host_library/exported")
     assert len(exported(MINE, "tsdr_")) == 18
 
 
-@needs_ref
-def test_status_codes_and_error_text_match_the_reference(tmp_path):
+def status_codes(path, plugin, tmp_path):
+    """Status codes and error texts of one library through a fixed sequence of calls, `plugin` as the source plugin."""
     raw = tmp_path / "iq.raw"
     synth.noise_iq(4096, seed=1).tofile(raw)
     nv, npl = VALUE_CB(lambda *a: None), PLOT_CB(lambda *a: None)
-    results = {}
-    for name, path in (("mine", MINE), ("ref", orc.REF_LIB_SO)):
-        lib = bind(path)
-        t = C.c_void_p()
-        lib.tsdr_init(C.byref(t), nv, npl, None)
-        lib.tsdr_setresolution(t, 525, 60.0); lib.tsdr_motionblur(t, 0.0); lib.tsdr_setgain(t, 0.5)
-        r = []
-        r.append(("readasync without plugin", lib.tsdr_readasync(t, FRAME_CB(lambda *a: None), None), lib.tsdr_getlasterrortext(t)))
-        r.append(("unload without plugin", lib.tsdr_unloadplugin(t), lib.tsdr_getlasterrortext(t)))
-        r.append(("getsamplerate without plugin", lib.tsdr_getsamplerate(t), lib.tsdr_getlasterrortext(t)))
-        r.append(("bad resolution", lib.tsdr_setresolution(t, 0, 60.0), lib.tsdr_getlasterrortext(t)))
-        r.append(("bad param id", lib.tsdr_setparameter_int(t, 99, 1), lib.tsdr_getlasterrortext(t)))
-        r.append(("good param", lib.tsdr_setparameter_int(t, 0, 1), lib.tsdr_getlasterrortext(t)))
-        r.append(("bad double id", lib.tsdr_setparameter_double(t, 7, 1.0), lib.tsdr_getlasterrortext(t)))
-        r.append(("bad motionblur", lib.tsdr_motionblur(t, 1.5), None))
-        r.append(("missing plugin file", lib.tsdr_loadplugin(t, b"/nonexistent/plugin.so", b""), lib.tsdr_getlasterrortext(t)))
-        r.append(("not a plugin", lib.tsdr_loadplugin(t, orc.PORT_SO.encode(), b""), lib.tsdr_getlasterrortext(t)))
-        r.append(("plugin param error", lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), f'"{raw}" 8000000'.encode()), lib.tsdr_getlasterrortext(t)))
-        r.append(("plugin ok", lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), f'"{raw}" 8000000 float'.encode()), lib.tsdr_getlasterrortext(t)))
-        r.append(("getsamplerate", lib.tsdr_getsamplerate(t), lib.tsdr_getlasterrortext(t)))
-        r.append(("sync too far", lib.tsdr_sync(t, 100000, 1), lib.tsdr_getlasterrortext(t)))
-        r.append(("sync ok", lib.tsdr_sync(t, 3, 3), lib.tsdr_getlasterrortext(t)))
-        r.append(("isrunning", lib.tsdr_isrunning(t), None))
-        r.append(("stop when idle", lib.tsdr_stop(t), lib.tsdr_getlasterrortext(t)))
-        r.append(("unload", lib.tsdr_unloadplugin(t), lib.tsdr_getlasterrortext(t)))
-        lib.tsdr_free(C.byref(t))
-        assert not t.value
-        results[name] = r
-    assert results["mine"] == results["ref"]
+    lib = bind(path)
+    t = C.c_void_p()
+    lib.tsdr_init(C.byref(t), nv, npl, None)
+    lib.tsdr_setresolution(t, 525, 60.0); lib.tsdr_motionblur(t, 0.0); lib.tsdr_setgain(t, 0.5)
+    r = []
+    r.append(("readasync without plugin", (lib.tsdr_readasync(t, FRAME_CB(lambda *a: None), None), lib.tsdr_getlasterrortext(t))))
+    r.append(("unload without plugin", (lib.tsdr_unloadplugin(t), lib.tsdr_getlasterrortext(t))))
+    r.append(("getsamplerate without plugin", (lib.tsdr_getsamplerate(t), lib.tsdr_getlasterrortext(t))))
+    r.append(("bad resolution", (lib.tsdr_setresolution(t, 0, 60.0), lib.tsdr_getlasterrortext(t))))
+    r.append(("bad param id", (lib.tsdr_setparameter_int(t, 99, 1), lib.tsdr_getlasterrortext(t))))
+    r.append(("good param", (lib.tsdr_setparameter_int(t, 0, 1), lib.tsdr_getlasterrortext(t))))
+    r.append(("bad double id", (lib.tsdr_setparameter_double(t, 7, 1.0), lib.tsdr_getlasterrortext(t))))
+    r.append(("bad motionblur", (lib.tsdr_motionblur(t, 1.5), None)))
+    r.append(("missing plugin file", (lib.tsdr_loadplugin(t, b"/nonexistent/plugin.so", b""), lib.tsdr_getlasterrortext(t))))
+    r.append(("not a plugin", (lib.tsdr_loadplugin(t, orc.PORT_SO.encode(), b""), lib.tsdr_getlasterrortext(t))))
+    bad = f'"{raw}" 8000000'
+    r.append(("plugin param error", (lib.tsdr_loadplugin(t, plugin.encode(), bad.encode()), forwarded(lib.tsdr_getlasterrortext(t), plugin_error_text(plugin, bad, tmp_path)))))
+    r.append(("plugin ok", (lib.tsdr_loadplugin(t, plugin.encode(), f'"{raw}" 8000000 float'.encode()), lib.tsdr_getlasterrortext(t))))
+    r.append(("getsamplerate", (lib.tsdr_getsamplerate(t), lib.tsdr_getlasterrortext(t))))
+    r.append(("sync too far", (lib.tsdr_sync(t, 100000, 1), lib.tsdr_getlasterrortext(t))))
+    r.append(("sync ok", (lib.tsdr_sync(t, 3, 3), lib.tsdr_getlasterrortext(t))))
+    r.append(("isrunning", (lib.tsdr_isrunning(t), None)))
+    r.append(("stop when idle", (lib.tsdr_stop(t), lib.tsdr_getlasterrortext(t))))
+    r.append(("unload", (lib.tsdr_unloadplugin(t), lib.tsdr_getlasterrortext(t))))
+    lib.tsdr_free(C.byref(t))
+    assert not t.value
+    return r
 
 
-@needs_ref
-def test_more_setter_scenarios_match_the_reference(tmp_path):
+def test_status_codes_and_error_text_match_the_reference(tmp_path):
+    assert_matches_reference("host_library/status_codes", status_codes(MINE, PLUGIN, tmp_path))
+
+
+def more_setter_scenarios(path, plugin, tmp_path):
     """Second sweep of the boundary (TSDRLibrary.c:136-262, 420-560): every setter with in-range, edge and out-of-range values, before
-    and after a plugin is loaded, repeated loads / unloads -- status codes and error texts identical to the compiled reference."""
+    and after a plugin is loaded, repeated loads / unloads."""
     raw = tmp_path / "iq.raw"
     synth.noise_iq(4096, seed=2).tofile(raw)
     nv, npl = VALUE_CB(lambda *a: None), PLOT_CB(lambda *a: None)
-    results = {}
-    for name, path in (("mine", MINE), ("ref", orc.REF_LIB_SO)):
-        lib = bind(path)
-        t = C.c_void_p()
-        lib.tsdr_init(C.byref(t), nv, npl, None)
-        r = []
-        txt = lambda: lib.tsdr_getlasterrortext(t)
-        r.append(("fresh: error text", None, txt()))
-        r.append(("isrunning fresh", lib.tsdr_isrunning(t), None))
-        r.append(("setbasefreq without plugin", lib.tsdr_setbasefreq(t, 100_000_000), txt()))
-        r.append(("setgain without plugin", lib.tsdr_setgain(t, 0.5), txt()))
-        r.append(("sync before resolution", lib.tsdr_sync(t, 1, 0), txt()))
-        for h, fv in ((525, 60.0), (1125, 59.94), (-3, 60.0), (525, 0.0), (525, -1.0), (1, 1.0)):
-            r.append((f"setresolution {h} {fv}", lib.tsdr_setresolution(t, h, fv), txt()))
-        lib.tsdr_setresolution(t, 525, 60.0)
-        for mb in (0.0, 0.5, 1.0, -0.1, 1.0001):
-            r.append((f"motionblur {mb}", lib.tsdr_motionblur(t, mb), txt()))
-        for pid in range(-1, 11):
-            r.append((f"param_int {pid}", lib.tsdr_setparameter_int(t, pid, 1), txt()))
-            lib.tsdr_setparameter_int(t, pid, 0)
-        for pid in range(-1, 4):
-            r.append((f"param_double {pid}", lib.tsdr_setparameter_double(t, pid, 0.25), txt()))
-        r.append(("plugin ok", lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), f'"{raw}" 8000000 float'.encode()), txt()))
-        r.append(("error text after success", None, txt()))
-        r.append(("plugin again", lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), f'"{raw}" 2000000 int8'.encode()), txt()))
-        r.append(("getsamplerate", lib.tsdr_getsamplerate(t), txt()))
-        for g in (0.0, 1.0, -0.5, 1.5):
-            r.append((f"setgain {g}", lib.tsdr_setgain(t, g), txt()))
-        r.append(("setbasefreq", lib.tsdr_setbasefreq(t, 433_920_000), txt()))
-        for px, d in ((0, 0), (5, 0), (5, 1), (5, 2), (5, 3), (5, 4), (-5, 0), (10_000_000, 2), (10_000_000, 0)):
-            r.append((f"sync {px} {d}", lib.tsdr_sync(t, px, d), txt()))
-        r.append(("bad plugin params keep", lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), b"nofile 0 float"), txt()))
-        r.append(("getsamplerate after failed load", lib.tsdr_getsamplerate(t), txt()))
-        r.append(("unload", lib.tsdr_unloadplugin(t), txt()))
-        r.append(("unload twice", lib.tsdr_unloadplugin(t), txt()))
-        r.append(("stop idle", lib.tsdr_stop(t), txt()))
-        lib.tsdr_free(C.byref(t))
-        results[name] = r
-    diff = [(a, b) for a, b in zip(results["mine"], results["ref"]) if a != b]
-    assert not diff, diff
+    lib = bind(path)
+    t = C.c_void_p()
+    lib.tsdr_init(C.byref(t), nv, npl, None)
+    r = []
+    txt = lambda: lib.tsdr_getlasterrortext(t)
+    r.append(("fresh: error text", (None, txt())))
+    r.append(("isrunning fresh", (lib.tsdr_isrunning(t), None)))
+    r.append(("setbasefreq without plugin", (lib.tsdr_setbasefreq(t, 100_000_000), txt())))
+    r.append(("setgain without plugin", (lib.tsdr_setgain(t, 0.5), txt())))
+    r.append(("sync before resolution", (lib.tsdr_sync(t, 1, 0), txt())))
+    for h, fv in ((525, 60.0), (1125, 59.94), (-3, 60.0), (525, 0.0), (525, -1.0), (1, 1.0)):
+        r.append((f"setresolution {h} {fv}", (lib.tsdr_setresolution(t, h, fv), txt())))
+    lib.tsdr_setresolution(t, 525, 60.0)
+    for mb in (0.0, 0.5, 1.0, -0.1, 1.0001):
+        r.append((f"motionblur {mb}", (lib.tsdr_motionblur(t, mb), txt())))
+    for pid in range(-1, 11):
+        r.append((f"param_int {pid}", (lib.tsdr_setparameter_int(t, pid, 1), txt())))
+        lib.tsdr_setparameter_int(t, pid, 0)
+    for pid in range(-1, 4):
+        r.append((f"param_double {pid}", (lib.tsdr_setparameter_double(t, pid, 0.25), txt())))
+    r.append(("plugin ok", (lib.tsdr_loadplugin(t, plugin.encode(), f'"{raw}" 8000000 float'.encode()), txt())))
+    r.append(("error text after success", (None, txt())))
+    r.append(("plugin again", (lib.tsdr_loadplugin(t, plugin.encode(), f'"{raw}" 2000000 int8'.encode()), txt())))
+    r.append(("getsamplerate", (lib.tsdr_getsamplerate(t), txt())))
+    for g in (0.0, 1.0, -0.5, 1.5):
+        r.append((f"setgain {g}", (lib.tsdr_setgain(t, g), txt())))
+    r.append(("setbasefreq", (lib.tsdr_setbasefreq(t, 433_920_000), txt())))
+    for px, d in ((0, 0), (5, 0), (5, 1), (5, 2), (5, 3), (5, 4), (-5, 0), (10_000_000, 2), (10_000_000, 0)):
+        r.append((f"sync {px} {d}", (lib.tsdr_sync(t, px, d), txt())))
+    r.append(("bad plugin params keep", (lib.tsdr_loadplugin(t, plugin.encode(), b"nofile 0 float"),
+                                         forwarded(txt(), plugin_error_text(plugin, "nofile 0 float", tmp_path)))))
+    r.append(("getsamplerate after failed load", (lib.tsdr_getsamplerate(t), txt())))
+    r.append(("unload", (lib.tsdr_unloadplugin(t), txt())))
+    r.append(("unload twice", (lib.tsdr_unloadplugin(t), txt())))
+    r.append(("stop idle", (lib.tsdr_stop(t), txt())))
+    lib.tsdr_free(C.byref(t))
+    return r
 
 
-@needs_ref
+def test_more_setter_scenarios_match_the_reference(tmp_path):
+    """Status codes and error texts identical to the compiled reference's in more_setter_scenarios."""
+    assert_matches_reference("host_library/more_setter_scenarios", more_setter_scenarios(MINE, PLUGIN, tmp_path))
+
+
 def test_readasync_without_gpu_fails_loudly(tmp_path):
     import torch
     if torch.cuda.is_available():
@@ -153,7 +174,7 @@ def test_readasync_without_gpu_fails_loudly(tmp_path):
     nv, npl = VALUE_CB(lambda *a: None), PLOT_CB(lambda *a: None)
     lib.tsdr_init(C.byref(t), nv, npl, None)
     lib.tsdr_setresolution(t, 525, 60.0)
-    assert lib.tsdr_loadplugin(t, orc.REF_RAWFILE_NOPACE_SO.encode(), f'"{raw}" 8000000 float'.encode()) == 0
+    assert lib.tsdr_loadplugin(t, PLUGIN.encode(), f'"{raw}" 8000000 float nopace'.encode()) == 0
     rc = lib.tsdr_readasync(t, FRAME_CB(lambda *a: None), None)
     assert rc == 6                                        # TSDR_CANNOT_OPEN_DEVICE
     assert b"no CPU fallback" in lib.tsdr_getlasterrortext(t)
@@ -162,9 +183,9 @@ def test_readasync_without_gpu_fails_loudly(tmp_path):
 
 
 @pytest.mark.gpu
-@needs_ref
-def test_host_library_end_to_end(tmp_path):
-    """tsdr_readasync + the reference's RawFile plugin on a file: delivered frames equal the oracle's stage-wise replay."""
+def test_host_library_end_to_end(tmp_path, monkeypatch):
+    """tsdr_readasync + a RawFile plugin on a file (this project's, in plain ten-symbol mode: float samples handed over
+    on the host like the reference's plugin does): delivered frames equal the oracle's stage-wise replay."""
     from tests.test_pipeline_gpu import run_oracle_stream
     O = orc.best()
     fs, h, fv = 2_000_000, 125, 60.0
@@ -177,6 +198,7 @@ def test_host_library_end_to_end(tmp_path):
     _, want = run_oracle_stream(O, [iq[k * items:(k + 1) * items] for k in range(nblk)], fs, h, fv)
     got = []
     os.environ["TSDR_NO_DROP"] = "1"
+    monkeypatch.setenv("TSDR_NO_RAW_SINK", "1")
     lib = bind(MINE)
     t = C.c_void_p()
     nv, npl = VALUE_CB(lambda *a: None), PLOT_CB(lambda *a: None)
@@ -185,7 +207,7 @@ def test_host_library_end_to_end(tmp_path):
     lib.tsdr_setresolution(t, h, fv); lib.tsdr_motionblur(t, 0.0); lib.tsdr_setgain(t, 0.5)
     for pid, v in ((0, 1), (1, 0), (6, 1)):
         lib.tsdr_setparameter_int(t, pid, v)
-    assert lib.tsdr_loadplugin(t, orc.REF_RAWFILE_SO.encode(), f'"{raw}" {int(fs)} float'.encode()) == 0
+    assert lib.tsdr_loadplugin(t, PLUGIN.encode(), f'"{raw}" {int(fs)} float'.encode()) == 0
     rc = []
     th = threading.Thread(target=lambda: rc.append(lib.tsdr_readasync(t, fcb, None)))
     th.start()

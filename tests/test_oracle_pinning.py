@@ -1,10 +1,9 @@
 """Pins the C restatement (oracle/tsdr_oracle.c) to the REAL reference.
 
-Two sources of truth:
-  * oracle/_ref/libtsdr_refharness.so -- the reference compiled in place from /root/reference (present in the build
-    container and, as a prebuilt binary, on the GPU box); every stage is compared bit-for-bit on seeded inputs;
-  * tests/golden/*.npz -- outputs of that same reference captured by tests/golden/make_golden.py, so the pin
-    survives on machines that have neither.
+Every scenario below runs a stage of an oracle on seeded inputs and lists what it observed.  The reference's own list --
+made by the compiled reference (oracle/_ref, built from the original sources) running the same scenario -- is stored in
+tests/golden/reference_outputs.json (tests/golden/make_reference_outputs.py), arrays as digests of their bits; the
+restatement has to reproduce it bit for bit.  tests/golden/*.npz pin a few paths with the arrays themselves.
 
 CPU only; no GPU, no product code.
 """
@@ -13,8 +12,7 @@ import pytest
 
 from oracle import oracle as orc
 from tempestsdr_b200 import synth
-
-needs_ref = pytest.mark.skipif(not orc.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
+from tests.test_golden import assert_matches_reference
 
 CFGS = {  # name: (samplerate, height, refreshrate)
     "cfg1": (8_000_000, 525, 60.0),
@@ -24,37 +22,42 @@ CFGS = {  # name: (samplerate, height, refreshrate)
     "odd": (2_400_000, 313, 59.94),
 }
 
-
-def bits(a):
-    a = np.ascontiguousarray(a)
-    return a.view(np.uint32 if a.dtype == np.float32 else np.uint64)
+SCENARIOS = {}
 
 
-def assert_same_bits(a, b, what=""):
-    assert a.shape == b.shape, what
-    assert np.array_equal(bits(a), bits(b)), f"{what}: {np.count_nonzero(bits(a) != bits(b))} of {a.size} differ"
+def scenario(fn):
+    """Registers fn(O, **params) -> [(label, value)] for make_reference_outputs.py."""
+    SCENARIOS[fn.__name__] = fn
+    return fn
 
 
-@needs_ref
-def test_am_demod():
-    P, R = orc.port(), orc.ref()
+def key(fn_name, /, **params):
+    return f"oracle_pinning/{fn_name}" + "".join(f"/{k}={v}" for k, v in sorted(params.items()))
+
+
+def check(fn, /, **params):
+    assert_matches_reference(key(fn.__name__, **params), fn(orc.port(), **params))
+
+
+@scenario
+def am_demod(O):
     iq = synth.noise_iq(50_001, seed=1)
     iq[:8] = [0, 0, 1e-30, 1e-30, 3e38, 1e38, -0.0, 0.0]
-    assert_same_bits(P.am_demod(iq), R.am_demod(iq), "am_demod")
-    assert P.am_demod(np.zeros(0, np.float32)).size == 0
+    return [("am_demod", O.am_demod(iq)), ("empty", O.am_demod(np.zeros(0, np.float32)).size)]
 
 
-@needs_ref
-@pytest.mark.parametrize("name", list(CFGS))
-@pytest.mark.parametrize("nearest", [False, True])
-def test_resample_stream(name, nearest):
+def test_am_demod():
+    check(am_demod)
+
+
+@scenario
+def resample_stream(O, name, nearest):
     fs, h, fv = CFGS[name]
-    P, R = orc.port(), orc.ref()
-    w, _, _ = R.geometry(fs, h, fv)
-    assert P.geometry(fs, h, fv) == R.geometry(fs, h, fv)
+    w, _, _ = O.geometry(fs, h, fv)
+    obs = [("geometry", O.geometry(fs, h, fv))]
     block = int(0.1 * fs / fv)
     rng = np.random.default_rng(7)
-    rp, rr = P.resampler(), R.resampler()
+    rs = O.resampler()
     up = w * h * fv
     # r == 2 exactly: the reference's loop emits one pixel fewer than it sizes the buffer for (dsp.c:262 vs
     # :288-297), so the last slot keeps what an earlier call left there -- zero while the buffer never moves,
@@ -65,80 +68,111 @@ def test_resample_stream(name, nearest):
         for k in range(14):
             n = block if (k % 5 or not ragged) else max(3, block // 3 + k)
             x = rng.uniform(0, 1, n).astype(np.float32)
-            a = rp.run(x, up, fs, nearest)
-            b = rr.run(x, up, fs, nearest)
+            a = rs.run(x, up, fs, nearest)
             if stale_tail and ragged:
-                assert rp.last_emitted == a.size - 1
-                a, b = a[:-1], b[:-1]
-            assert_same_bits(a, b, f"resample {name} block {k}")
-            assert rp.state == rr.state
+                if O.kind == "port":
+                    assert rs.last_emitted == a.size - 1
+                a = a[:-1]
+            obs += [(f"resample {name} ragged={ragged} block {k}", a), (f"state after block {k}", rs.state)]
+    return obs
 
 
-@needs_ref
-@pytest.mark.parametrize("ratio", [0.37, 0.9999, 1.0, 1.5, 2.0, 3.25])
-def test_resample_general_ratio(ratio):
-    P, R = orc.port(), orc.ref()
+@pytest.mark.parametrize("name", list(CFGS))
+@pytest.mark.parametrize("nearest", [False, True])
+def test_resample_stream(name, nearest):
+    check(resample_stream, name=name, nearest=nearest)
+
+
+@scenario
+def resample_general_ratio(O, ratio):
     rng = np.random.default_rng(11)
-    rp, rr = P.resampler(), R.resampler()
+    rs, lead = O.resampler(), orc.port().resampler()
+    obs = []
     for k in range(9):
         x = rng.standard_normal(1000 + 37 * k).astype(np.float32)
-        a, b = rp.run(x, ratio * 1e6, 1e6), rr.run(x, ratio * 1e6, 1e6)
+        a = rs.run(x, ratio * 1e6, 1e6)
+        lead.run(x, ratio * 1e6, 1e6)
         # when (size-offset)*r lands exactly on an integer the loop writes one pixel fewer than output_samples and,
-        # the buffer having grown, the reference's last slot is uninitialised heap: exclude exactly that slot
-        m = min(rp.last_emitted, a.size)
-        a, b = a[:m], b[:m]
-        assert_same_bits(a, b, f"ratio {ratio} block {k}")
-        assert rp.state == rr.state
+        # the buffer having grown, the reference's last slot is uninitialised heap: exclude exactly that slot (the
+        # restatement, run in step, tells how many pixels the loop wrote)
+        obs += [(f"ratio {ratio} block {k}", a[:min(lead.last_emitted, a.size)]), (f"state after block {k}", rs.state)]
+    return obs
 
 
-@needs_ref
-def test_dropcomp():
-    P, R = orc.port(), orc.ref()
+@pytest.mark.parametrize("ratio", [0.37, 0.9999, 1.0, 1.5, 2.0, 3.25])
+def test_resample_general_ratio(ratio):
+    check(resample_general_ratio, ratio=ratio)
+
+
+@scenario
+def dropcomp(O):
     rng = np.random.default_rng(3)
-    for _ in range(400):
+    obs = []
+    for i in range(400):
         block = int(rng.integers(1, 5000))
         diff = int(rng.integers(0, 3 * block))
         off = int(rng.integers(-4 * block, 4 * block))
         size = int(rng.integers(0, 4 * block))
-        assert P.dropcomp_shift_with(diff, block, off) == R.dropcomp_shift_with(diff, block, off)
-        assert P.dropcomp_will_drop_all(diff, size, block) == R.dropcomp_will_drop_all(diff, size, block)
-        for ok in (True, False):
-            assert P.dropcomp_add(diff, size, block, ok) == R.dropcomp_add(diff, size, block, ok)
+        obs += [(f"{i} shift_with", O.dropcomp_shift_with(diff, block, off)),
+                (f"{i} will_drop_all", O.dropcomp_will_drop_all(diff, size, block))]
+        obs += [(f"{i} add ring_accepts={ok}", O.dropcomp_add(diff, size, block, ok)) for ok in (True, False)]
+    return obs
 
 
-@needs_ref
-def test_frame_stage_pieces():
-    P, R = orc.port(), orc.ref()
+def test_dropcomp():
+    check(dropcomp)
+
+
+@scenario
+def frame_stage_pieces(O):
     w, h = 507, 525
     f = synth.video_like_frame(w, h, seed=5, shift_x=100, shift_y=40)
     f[1234] = 512.0; f[99] = -300.0     # marker values must pass through auto-gain
-    sp, sr = orc.Autogain(0, 0, 1), orc.Autogain(0, 0, 1)
-    for _ in range(3):
-        a = P.autogain(sp, f, 0.1); b = R.autogain(sr, f, 0.1)
-        assert_same_bits(a, b, "autogain")
-        assert (sp.lastmax, sp.lastmin, sp.snr) == (sr.lastmax, sr.lastmin, sr.snr)
-    s1 = np.zeros(w * h, np.float32); s2 = np.zeros(w * h, np.float32)
+    obs = []
+    st = orc.Autogain(0, 0, 1)
+    for k in range(3):
+        obs += [(f"autogain {k}", O.autogain(st, f, 0.1)), (f"autogain state {k}", (st.lastmax, st.lastmin, st.snr))]
+    s = np.zeros(w * h, np.float32)
     for c in (0.0, 0.3, 0.97):
-        P.timelowpass(c, f, s1); R.timelowpass(c, f, s2)
-        assert_same_bits(s1, s2, f"timelowpass {c}")
-    (wa, ha), (wb, hb) = P.average_v_h(f, w, h), R.average_v_h(f, w, h)
-    assert_same_bits(wa, wb, "colsum"); assert_same_bits(ha, hb, "rowsum")
+        O.timelowpass(c, f, s)
+        obs.append((f"timelowpass {c}", s.copy()))
+    wa, ha = O.average_v_h(f, w, h)
+    obs += [("colsum", wa), ("rowsum", ha)]
     for n in (1, 2, 3, 4, 5, 6, 17, 507):
         s = np.random.default_rng(n).uniform(0, 5, n).astype(np.float32)
-        assert_same_bits(P.gaussianblur(s), R.gaussianblur(s), f"gauss n={n}")
+        obs.append((f"gauss n={n}", O.gaussianblur(s)))
     for strip in (wa, ha):
         for size in (5, 13, strip.size // 3):
-            assert P.findbestfit(strip, float(strip.sum()), size) == R.findbestfit(strip, float(strip.sum()), size)
-    a, b = orc.Sweetspot(), orc.Sweetspot()
+            obs.append((f"findbestfit {strip.size} {size}", O.findbestfit(strip, float(strip.sum()), size)))
+    sw = orc.Sweetspot()
     for k in range(6):
-        strip = np.roll(wa, 17 * k)
-        o1 = P.findthesweetspot(a, strip, int(w * 0.05), 0.9)
-        o2 = R.findthesweetspot(b, strip, int(w * 0.05), 0.9)
-        assert a.astuple() == b.astuple()
-        assert_same_bits(o1, o2, "sweetspot strip")
+        o = O.findthesweetspot(sw, np.roll(wa, 17 * k), int(w * 0.05), 0.9)
+        obs += [(f"sweetspot state {k}", sw.astuple()), (f"sweetspot strip {k}", o)]
+    return obs
 
 
-@needs_ref
+def test_frame_stage_pieces():
+    check(frame_stage_pieces)
+
+
+PP_FIELDS = ("avg_speed", "pll_state", "lastmax", "lastmin", "refreshrate_after", "width_after", "pll_callback_fired",
+             "autogain_callback_fired", "autogain_cb_min", "autogain_cb_max", "snr")
+
+
+@scenario
+def post_process_sequence(O, lpbs, aap, autoshift, pll, mb):
+    fs, hgt, fv = CFGS["cfg1"]
+    pp = O.postprocessor(fs, hgt, fv, autoshift, pll)
+    w, _, _ = O.geometry(fs, hgt, fv)
+    obs = []
+    for k in range(9):
+        f = synth.video_like_frame(w, hgt, seed=k, shift_x=60 + 9 * k, shift_y=20 + 3 * k)
+        a, r = pp.run(f, w, hgt, mb, 0.1, lpbs, aap)
+        obs += [(f"frame {k}", a), (f"sync {k}", (r.x.astuple(), r.y.astuple()))]
+        obs += [(f"{fld} {k}", getattr(r, fld)) for fld in PP_FIELDS]
+    return obs
+
+
 @pytest.mark.parametrize("lpbs,aap,autoshift,pll,mb", [
     (1, 0, 1, 0, 0.0),   # GUI default minus PLL
     (1, 0, 1, 1, 0.0),   # GUI default
@@ -149,75 +183,74 @@ def test_frame_stage_pieces():
     (1, 0, 0, 0, 0.0),   # green lines on a copy
 ])
 def test_post_process_sequence(lpbs, aap, autoshift, pll, mb):
-    P, R = orc.port(), orc.ref()
-    fs, hgt, fv = CFGS["cfg1"]
-    pp, pr = P.postprocessor(fs, hgt, fv, autoshift, pll), R.postprocessor(fs, hgt, fv, autoshift, pll)
-    w, _, _ = R.geometry(fs, hgt, fv)
-    for k in range(9):
-        f = synth.video_like_frame(w, hgt, seed=k, shift_x=60 + 9 * k, shift_y=20 + 3 * k)
-        a, ra = pp.run(f, w, hgt, mb, 0.1, lpbs, aap)
-        b, rb = pr.run(f, w, hgt, mb, 0.1, lpbs, aap)
-        assert_same_bits(a, b, f"frame {k}")
-        for fld in ("avg_speed", "pll_state", "lastmax", "lastmin", "refreshrate_after", "width_after",
-                    "pll_callback_fired", "autogain_callback_fired", "autogain_cb_min", "autogain_cb_max"):
-            assert getattr(ra, fld) == getattr(rb, fld), (k, fld)
-        assert ra.x.astuple() == rb.x.astuple() and ra.y.astuple() == rb.y.astuple()
-        assert ra.snr == rb.snr or (np.isnan(ra.snr) and np.isnan(rb.snr))
+    check(post_process_sequence, lpbs=lpbs, aap=aap, autoshift=autoshift, pll=pll, mb=mb)
 
 
-@needs_ref
-def test_post_process_resize_and_flag_flip():
-    P, R = orc.port(), orc.ref()
-    pp, pr = P.postprocessor(8_000_000, 525, 60.0), R.postprocessor(8_000_000, 525, 60.0)
+@scenario
+def post_process_resize_and_flag_flip(O):
+    pp = O.postprocessor(8_000_000, 525, 60.0)
     shapes = [(200, 100, 1), (200, 100, 1), (150, 120, 1), (150, 120, 0), (300, 200, 0), (200, 100, 1)]
+    obs = []
     for k, (w, h, lpbs) in enumerate(shapes):
         f = synth.video_like_frame(w, h, seed=40 + k, shift_x=11, shift_y=7)
-        a, ra = pp.run(f, w, h, 0.25, 0.1, lpbs, 0)
-        b, rb = pr.run(f, w, h, 0.25, 0.1, lpbs, 0)
-        assert_same_bits(a, b, f"resize step {k}")
+        obs.append((f"resize step {k}", pp.run(f, w, h, 0.25, 0.1, lpbs, 0)[0]))
+    return obs
 
 
-@needs_ref
+def test_post_process_resize_and_flag_flip():
+    check(post_process_resize_and_flag_flip)
+
+
+@scenario
+def fft(O, logn):
+    x = synth.noise_iq(1 << logn, seed=logn)
+    return [(f"fft 2^{logn} inv={inv}", O.fft(x, inv)) for inv in (False, True)]
+
+
 @pytest.mark.parametrize("logn", [0, 1, 2, 3, 7, 12, 16])
 def test_fft(logn):
-    P, R = orc.port(), orc.ref()
-    n = 1 << logn
-    x = synth.noise_iq(n, seed=logn)
-    for inv in (False, True):
-        assert_same_bits(P.fft(x, inv), R.fft(x, inv), f"fft 2^{logn} inv={inv}")
+    check(fft, logn=logn)
 
 
-@needs_ref
-@pytest.mark.parametrize("size", [1, 5, 1000, 4096, 70_001])
-def test_autocorrelation_and_xcorr(size):
-    P, R = orc.port(), orc.ref()
+@scenario
+def autocorrelation_and_xcorr(O, size):
     x = np.abs(synth.noise_iq(size, seed=size)[:size])
-    assert_same_bits(P.autocorrelation(x), R.autocorrelation(x), "autocorrelation")
+    obs = [("autocorrelation", O.autocorrelation(x))]
     if size >= 4:
         a = synth.noise_iq(size, seed=1); b = synth.noise_iq(size, seed=2)
-        n = P.fft_getrealsize(size)
-        assert_same_bits(P.crosscorrelation(a, b)[: 2 * n], R.crosscorrelation(a, b)[: 2 * n], "xcorr")
+        n = orc.port().fft_getrealsize(size)
+        obs.append(("xcorr", O.crosscorrelation(a, b)[: 2 * n]))
+    return obs
 
 
-@needs_ref
-def test_framerate_detector_plots():
-    P, R = orc.port(), orc.ref()
+@pytest.mark.parametrize("size", [1, 5, 1000, 4096, 70_001])
+def test_autocorrelation_and_xcorr(size):
+    check(autocorrelation_and_xcorr, size=size)
+
+
+@scenario
+def framerate_detector_plots(O):
+    P = orc.port()                 # the capture size and the demodulated input come from the restatement (pinned above)
     fs = 2_000_000
     size = P.framerate_capture_size(fs)
-    dp, dr = P.framerate_detector(), R.framerate_detector()
+    det = O.framerate_detector()
+    obs = []
     for k in range(3):
-        iq = synth.video_like_iq(size, fs, 400, 200, 50.0, seed=k)
-        x = P.am_demod(iq)
-        (fo, fp), (lo, lp), c = dp.run(fs, x)
-        (fo2, fp2), (lo2, lp2), c2 = dr.run(fs, x)
-        assert (fo, lo, c) == (fo2, lo2, c2) and c == k + 1
-        assert P.framerate_windows(fs) == (fo, fo + fp.size, lo, lo + lp.size)
-        assert_same_bits(fp, fp2, "frame plot"); assert_same_bits(lp, lp2, "line plot")
+        x = P.am_demod(synth.video_like_iq(size, fs, 400, 200, 50.0, seed=k))
+        (fo, fp), (lo, lp), c = det.run(fs, x)
+        assert c == k + 1
+        if O.kind == "port":
+            assert P.framerate_windows(fs) == (fo, fo + fp.size, lo, lo + lp.size)
+        obs += [(f"offsets and calls {k}", (fo, lo, c)), (f"frame plot {k}", fp), (f"line plot {k}", lp)]
+    return obs
 
 
-@needs_ref
-def test_superbandwidth_stitch():
-    P, R = orc.port(), orc.ref()
+def test_framerate_detector_plots():
+    check(framerate_detector_plots)
+
+
+@scenario
+def superbandwidth_stitch(O):
     fs, fv = 400_000, 50.0
     sif = int(fs / fv)             # 8000 samples per frame, does not divide 2^k
     pairs = 10 * sif               # 80000 -> N = 65536
@@ -227,14 +260,15 @@ def test_superbandwidth_stitch():
         seg = base[2 * lag: 2 * (lag + pairs)].copy()
         seg += synth.noise_iq(pairs, seed=100 + i, scale=0.01)
         hops.append(seg)
-    for i in range(1, 4):
-        n2 = 2 * P.fft_getrealsize(pairs)
-        assert P.superb_bestfit(hops[0][:n2], hops[i][:n2], sif) == R.superb_bestfit(hops[0][:n2], hops[i][:n2], sif)
-    d = hops[1][:4096]
-    assert_same_bits(P.complex_to_abs_diff(d), R.complex_to_abs_diff(d), "abs diff")
-    (a, oa), (b, ob) = P.superb_ondataready(hops, sif), R.superb_ondataready(hops, sif)
-    assert list(oa) == list(ob)
-    assert_same_bits(a, b, "stitched")
+    n2 = 2 * orc.port().fft_getrealsize(pairs)
+    obs = [(f"bestfit hop {i}", O.superb_bestfit(hops[0][:n2], hops[i][:n2], sif)) for i in range(1, 4)]
+    obs.append(("abs diff", O.complex_to_abs_diff(hops[1][:4096])))
+    out, offs = O.superb_ondataready(hops, sif)
+    return obs + [("offsets", list(offs)), ("stitched", out)]
+
+
+def test_superbandwidth_stitch():
+    check(superbandwidth_stitch)
 
 
 def test_pixel_rule():

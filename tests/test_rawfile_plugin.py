@@ -3,7 +3,9 @@
 CPU: the plugin is an ordinary ten-symbol TSDR plugin -- same parameter errors as the reference's TSDRPlugin_RawFile, the
 same floats through the ordinary callback (including what is delivered around the end of the file).
 GPU: the device conversion is bit-identical to the plugin's host expressions for EVERY 8- and 16-bit code, and a run
-through the host library with the raw sink delivers bit-identical frames to a run with the reference's own plugin."""
+through the host library with the raw sink delivers bit-identical frames to a run that converts on the host, fed the
+floats the reference's own plugin delivers for the same recording.
+What the reference's plugin did is recorded in tests/golden/reference_outputs.json (tests/golden/make_reference_outputs.py)."""
 import ctypes as C
 import os
 import subprocess
@@ -15,11 +17,11 @@ import pytest
 
 from oracle import oracle as orc
 from tempestsdr_b200 import synth
+from tests.test_golden import assert_matches_reference, reference_outputs
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PLUGIN = os.path.join(ROOT, "tempestsdr_b200", "lib", "TSDRPlugin_RawFileGPU.so")
 MINE = os.path.join(ROOT, "tempestsdr_b200", "lib", "libTSDRLibrary.so")
-needs_ref = pytest.mark.skipif(not orc.have_ref(), reason="compiled reference (oracle/_ref) not present")
 PLUGIN_CB = C.CFUNCTYPE(None, C.POINTER(C.c_float), C.c_uint64, C.c_void_p, C.c_int64)
 TEN = ["tsdrplugin_init", "tsdrplugin_getsamplerate", "tsdrplugin_getName", "tsdrplugin_setsamplerate", "tsdrplugin_setbasefreq",
        "tsdrplugin_stop", "tsdrplugin_setgain", "tsdrplugin_readasync", "tsdrplugin_getlasterrortext", "tsdrplugin_cleanup"]
@@ -73,8 +75,11 @@ def test_plugin_exports_the_plugin_abi():
     assert b"Raw" in name.value
 
 
-@pytest.mark.parametrize("params", ["", "somefile", "somefile 0 float", "somefile 8000000", "somefile 8000000 int12",
-                                    "somefile -5 int8", "somefile 2000000000 float", "'some file' 8000000 float"])
+PARAMS = ["", "somefile", "somefile 0 float", "somefile 8000000", "somefile 8000000 int12", "somefile -5 int8",
+          "somefile 2000000000 float", "'some file' 8000000 float"]
+
+
+@pytest.mark.parametrize("params", PARAMS)
 def test_parameter_errors_match_the_reference_plugin(params):
     mine = bind_plugin(PLUGIN)
     rc = mine.tsdrplugin_init(C.create_string_buffer(params.encode()))
@@ -82,39 +87,44 @@ def test_parameter_errors_match_the_reference_plugin(params):
     assert (rc == 0) == ok_expected
     assert rc in (0, 4)                                    # TSDR_PLUGIN_PARAMETERS_WRONG
     assert (mine.tsdrplugin_getlasterrortext() is None) == (rc == 0)
-    if orc.have_ref():
-        ref = bind_plugin(orc.REF_RAWFILE_NOPACE_SO)
-        assert ref.tsdrplugin_init(C.create_string_buffer(params.encode())) == rc
+    assert reference_outputs("rawfile_plugin/init_rc")[PARAMS.index(params)] == rc
     assert mine.tsdrplugin_init(C.create_string_buffer(b"f 1000 int8 nopace block=7")) == 4      # odd block
     assert mine.tsdrplugin_init(C.create_string_buffer(b"f 1000 int8 bogus")) == 4
     assert mine.tsdrplugin_init(C.create_string_buffer(b"f 1000 int8 nopace block=4096")) == 0
     assert mine.tsdrplugin_getsamplerate() == 1000
 
 
-@pytest.mark.parametrize("dtype,name", [(np.int8, "int8"), (np.uint8, "uint8"), (np.int16, "int16"), (np.uint16, "uint16"), (np.float32, "float")])
-def test_plugin_without_a_sink_is_an_ordinary_rawfile_plugin(tmp_path, dtype, name):
-    """No raw sink offered (as under the reference library): host conversion, float callback, and the reference's behaviour
-    at the end of the file -- the block buffer is delivered as it stands (fresh head, stale tail), then the file restarts."""
+def one_and_a_half_blocks(dtype, path):
+    """A recording of one and a half plugin blocks of seeded samples; returns the samples."""
     items = 512 * 1024
     rng = np.random.default_rng(5)
-    n = items + items // 2                                 # one and a half blocks
+    n = items + items // 2
     if dtype == np.float32:
         data = rng.standard_normal(n).astype(np.float32)
     else:
         info = np.iinfo(dtype)
         data = rng.integers(info.min, info.max + 1, n, dtype=np.int64).astype(dtype)
+    data.tofile(path)
+    return data
+
+
+DTYPES = [(np.int8, "int8"), (np.uint8, "uint8"), (np.int16, "int16"), (np.uint16, "uint16"), (np.float32, "float")]
+
+
+@pytest.mark.parametrize("dtype,name", DTYPES)
+def test_plugin_without_a_sink_is_an_ordinary_rawfile_plugin(tmp_path, dtype, name):
+    """No raw sink offered (as under the reference library): host conversion, float callback, and the reference's behaviour
+    at the end of the file -- the block buffer is delivered as it stands (fresh head, stale tail), then the file restarts."""
+    items = 512 * 1024
     raw = tmp_path / f"iq.{name}"
-    data.tofile(raw)
+    data = one_and_a_half_blocks(dtype, raw)
     mine = collect_blocks(PLUGIN, f'"{raw}" 8000000 {name} nopace', 4)
     conv = reference_floats(data)
     second = np.concatenate([conv[items:], conv[items // 2: items]])       # 0.5 block fresh + the stale tail of block 1
     want = [conv[:items], second, conv[:items], second]
     for k in range(4):
         assert np.array_equal(mine[k].view(np.uint32), want[k].view(np.uint32)), f"block {k}"
-    if orc.have_ref():
-        ref = collect_blocks(orc.REF_RAWFILE_NOPACE_SO, f'"{raw}" 8000000 {name}', 4)
-        for k in range(4):
-            assert np.array_equal(mine[k].view(np.uint32), ref[k].view(np.uint32)), f"block {k} vs the reference plugin"
+    assert_matches_reference(f"rawfile_plugin/blocks/{name}", [(f"block {k}", mine[k]) for k in range(4)])
 
 
 # ------------------------------------------------------------------------------------------------------------ GPU
@@ -167,28 +177,36 @@ def _run_host_library(plugin_path, params, fs, h, fv, nframes, env=None):
             else: os.environ[k] = v
 
 
-@pytest.mark.gpu
-@needs_ref
-@pytest.mark.parametrize("dtype,name", [(np.int8, "int8"), (np.uint8, "uint8"), (np.int16, "int16")])
-def test_raw_sink_run_equals_a_run_with_the_reference_plugin(tmp_path, dtype, name):
-    """Same recording, same library: (a) the reference's RawFile plugin converting on the host, (b) the GPU-aware plugin
-    with its raw sink (samples cross PCIe as integers), (c) the GPU-aware plugin with the sink withheld.  Frames agree bit
-    for bit -- the device conversion is the host conversion."""
+def quantised_recording(dtype, path):
+    """Six plugin blocks of video-like IQ at 2 MS/s, quantised to `dtype`; returns (fs, h, fv)."""
     fs, h, fv = 2_000_000, 125, 60.0
-    O = orc.best()
-    w, _, _ = O.geometry(fs, h, fv)
+    w, _, _ = orc.port().geometry(fs, h, fv)
     items = 512 * 1024
     iq = synth.video_like_iq(6 * items // 2, fs, w, h, fv, seed=77)
     info = np.iinfo(dtype)
     scale = 100.0 if dtype != np.int16 else 20000.0
     q = np.clip(np.round(iq / np.abs(iq).max() * scale) + (128 if dtype == np.uint8 else 0), info.min, info.max).astype(dtype)
+    q.tofile(path)
+    return fs, h, fv
+
+
+SINK_DTYPES = [(np.int8, "int8"), (np.uint8, "uint8"), (np.int16, "int16")]
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("dtype,name", SINK_DTYPES)
+def test_raw_sink_run_equals_a_run_with_the_reference_plugin(tmp_path, dtype, name):
+    """Same recording, same library: (a) the GPU-aware plugin with the sink withheld, converting on the host -- the floats it
+    hands over for the whole recording are the reference RawFile plugin's, bit for bit -- and (b) the GPU-aware plugin with
+    its raw sink (samples cross PCIe as integers).  Frames agree bit for bit -- the device conversion is the host
+    conversion."""
     raw = tmp_path / f"iq.{name}"
-    q.tofile(raw)
+    fs, h, fv = quantised_recording(dtype, raw)
+    blocks = collect_blocks(PLUGIN, f'"{raw}" {fs} {name} nopace', 6)
+    assert_matches_reference(f"rawfile_plugin/recording/{name}", [(f"block {k}", b) for k, b in enumerate(blocks)])
     nframes = 12
-    a = _run_host_library(orc.REF_RAWFILE_NOPACE_SO, f'"{raw}" {fs} {name}', fs, h, fv, nframes)
+    a = _run_host_library(PLUGIN, f'"{raw}" {fs} {name} nopace', fs, h, fv, nframes, env={"TSDR_NO_RAW_SINK": "1"})
     b = _run_host_library(PLUGIN, f'"{raw}" {fs} {name} nopace', fs, h, fv, nframes)
-    c = _run_host_library(PLUGIN, f'"{raw}" {fs} {name} nopace', fs, h, fv, nframes, env={"TSDR_NO_RAW_SINK": "1"})
-    assert min(len(a), len(b), len(c)) >= nframes
+    assert min(len(a), len(b)) >= nframes
     for k in range(nframes):
-        assert np.array_equal(a[k].view(np.uint32), b[k].view(np.uint32)), f"frame {k}: raw sink vs reference plugin"
-        assert np.array_equal(a[k].view(np.uint32), c[k].view(np.uint32)), f"frame {k}: host conversion vs reference plugin"
+        assert np.array_equal(a[k].view(np.uint32), b[k].view(np.uint32)), f"frame {k}: raw sink vs host conversion"
