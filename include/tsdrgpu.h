@@ -332,6 +332,36 @@ TSDRGPU_API int  tsdrgpu_superb_mgpu_stitch(tsdrgpu_superb_mgpu_t *g, void *stre
 TSDRGPU_API int  tsdrgpu_superb_mgpu_stream_window(tsdrgpu_superb_mgpu_t *g, float **d_stream);
 TSDRGPU_API int  tsdrgpu_superb_mgpu_lags(tsdrgpu_superb_mgpu_t *g, void *stream, int *h_lags, uint32_t *h_status);
 
+/* ---------------------------------------------------------------------------- tuner (digital down-converter)
+ * Not in the reference: picks one sub-band out of a wideband capture ahead of the pixel path (DESIGN.md section 5.6).  Input
+ * pair n (absolute index since the last reset, dropped pairs counted) is mixed by e^{-2 pi i offset n / fs} with the integer
+ * phase n * phase_inc mod 2^64, low-passed by a real linear-phase FIR and decimated by D: output m is
+ * z[m] = sum_k h[k] x~[mD - k], x~ = the mixed input with zeros before the first sample and over every drop, produced for every
+ * m with mD inside a block (outputs whose mD falls into a drop are withheld and counted as the output drop count).
+ * Configuration rules: decimation in 1..64, ntaps odd in 3..1023 (0 = 16 * ceil(fs / bandwidth) + 1, at most 1023),
+ * fs % decimation == 0, 0 < bandwidth_hz <= fs / decimation, |offset_hz| + bandwidth_hz / 2 <= fs / 2; anything else is
+ * TSDRGPU_EINVAL with a text naming the rule.  Filter: scipy.signal.firwin(ntaps, bandwidth_hz / 2, window=('kaiser', 7.857),
+ * fs=fs) designed in double, stored as float32. */
+typedef struct tsdrgpu_tuner tsdrgpu_tuner_t;
+/* host-only: validates and returns the float32 taps (cap entries at least) and the phase increment round(offset / fs * 2^64)
+ * (two's complement).  taps / ntaps_out / phase_inc may be NULL (validation only). */
+TSDRGPU_API int tsdrgpu_tuner_design(uint32_t fs, double offset_hz, double bandwidth_hz, int decimation, int ntaps, float *taps, int cap,
+                                     int *ntaps_out, uint64_t *phase_inc);
+/* host-only: outputs of a block of `pairs` input pairs preceded by `dropped` lost pairs, the stream being at absolute index
+ * `position` before the loss: *out_dropped = ceil((position + dropped) / D) - ceil(position / D),
+ * *out_pairs = ceil((position + dropped + pairs) / D) - ceil((position + dropped) / D). */
+TSDRGPU_API int tsdrgpu_tuner_out_pairs(uint64_t position, uint64_t pairs, uint64_t dropped, int decimation, uint64_t *out_pairs,
+                                        uint64_t *out_dropped);
+TSDRGPU_API int  tsdrgpu_tuner_create(tsdrgpu_ctx_t *ctx, tsdrgpu_tuner_t **t);
+TSDRGPU_API void tsdrgpu_tuner_destroy(tsdrgpu_tuner_t *t);
+/* (re)design the filter and reset; synchronises the device */
+TSDRGPU_API int  tsdrgpu_tuner_configure(tsdrgpu_tuner_t *t, uint32_t fs, double offset_hz, double bandwidth_hz, int decimation, int ntaps);
+TSDRGPU_API int  tsdrgpu_tuner_reset(tsdrgpu_tuner_t *t, void *stream);      /* position 0, history zero */
+/* d_iq: `pairs` interleaved I,Q pairs; d_out receives *out_pairs pairs (at most ceil(pairs / D) + 1).  Asynchronous: the counts
+ * come from host state (tsdrgpu_tuner_out_pairs), the device history of the last ntaps - 1 mixed samples is updated in stream order. */
+TSDRGPU_API int  tsdrgpu_tuner_run(tsdrgpu_tuner_t *t, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before, float *d_out,
+                                   uint64_t *out_pairs, uint64_t *out_dropped);
+
 /* ---------------------------------------------------------------------------- a1, a3, a5, a16, a17  streaming pipeline
  * replaces the body of process() (TSDRLibrary.c:264-298), decimatingthread / postprocessingthread /
  * videodecodingthread (TSDRLibrary.c:300-418) with their three rings (circbuff.c), dsp_dropped_compensation_*
@@ -391,6 +421,14 @@ TSDRGPU_API int  tsdrgpu_pipeline_flush(tsdrgpu_pipeline_t *p);            /* wa
 TSDRGPU_API int  tsdrgpu_pipeline_set_param_int(tsdrgpu_pipeline_t *p, int id, uint32_t value);
 TSDRGPU_API int  tsdrgpu_pipeline_set_resolution(tsdrgpu_pipeline_t *p, int height, double refreshrate);
 TSDRGPU_API int  tsdrgpu_pipeline_set_samplerate(tsdrgpu_pipeline_t *p, uint32_t samplerate);
+/* The tuner ahead of the pixel path (see tsdrgpu_tuner_*): every block is shifted by offset_hz, low-passed and decimated by
+ * `decimation` right after it reaches the device (any ingest format), and the rest of the pipeline runs at samplerate /
+ * decimation (geometry, decimator blocks, frame-rate detector, plots).  bandwidth_hz <= 0 switches it off (the default).
+ * Checked against the current rate at once (TSDRGPU_EINVAL + text); takes effect at the next process() call, which then starts
+ * over: tuner at position 0 with a zero history, samples and pixels waiting at the old rate discarded, resampler, frame stage
+ * and frame-rate detector reset.  Superbandwidth mode bypasses the tuner and resumes it, reset, when it ends.
+ * set_samplerate re-designs the taps for the new rate and rejects a rate the current tuning cannot take. */
+TSDRGPU_API int  tsdrgpu_pipeline_set_tuner(tsdrgpu_pipeline_t *p, double offset_hz, double bandwidth_hz, int decimation, int ntaps);
 /* superbandwidth mode (PARAM_AUTOCORR_SUPERRESOLUTION = 1; superb_run, superbandwidth.c:179-254) retunes the front end
  * between hops through this callback; without it the hops are recorded at one frequency */
 TSDRGPU_API int  tsdrgpu_pipeline_set_retune(tsdrgpu_pipeline_t *p, tsdrgpu_retune_cb cb);

@@ -147,6 +147,16 @@ _SIGS = {
     "tsdrgpu_pipeline_set_param_int": (C.c_int, [C.c_void_p, C.c_int, C.c_uint32]),
     "tsdrgpu_pipeline_set_resolution": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),
     "tsdrgpu_pipeline_set_samplerate": (C.c_int, [C.c_void_p, C.c_uint32]),
+    "tsdrgpu_pipeline_set_tuner": (C.c_int, [C.c_void_p, C.c_double, C.c_double, C.c_int, C.c_int]),
+    "tsdrgpu_tuner_design": (C.c_int, [C.c_uint32, C.c_double, C.c_double, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                       C.POINTER(C.c_int), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_tuner_out_pairs": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_tuner_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "tsdrgpu_tuner_destroy": (None, [C.c_void_p]),
+    "tsdrgpu_tuner_configure": (C.c_int, [C.c_void_p, C.c_uint32, C.c_double, C.c_double, C.c_int, C.c_int]),
+    "tsdrgpu_tuner_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tsdrgpu_tuner_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                                    C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
     "tsdrgpu_pipeline_set_retune": (C.c_int, [C.c_void_p, RETUNE_CB]),
     "tsdrgpu_pipeline_set_motionblur": (C.c_int, [C.c_void_p, C.c_float]),
     "tsdrgpu_pipeline_set_host_registration": (C.c_int, [C.c_void_p, C.c_int]),

@@ -183,6 +183,74 @@ class Context:
     def framerate_detector(self) -> "FrameRateDetector":
         return FrameRateDetector(self)
 
+    def tuner(self) -> "Tuner":
+        return Tuner(self)
+
+
+def tuner_design(fs: int, offset_hz: float, bandwidth_hz: float, decimation: int = 1, ntaps: int = 0) -> Tuple[np.ndarray, int]:
+    """tsdrgpu_tuner_design (host only): the float32 taps and the 64-bit phase increment round(offset / fs * 2^64) (as an
+    unsigned integer) the tuner uses for this configuration.  Raises TsdrGpuError naming the violated rule."""
+    taps = np.zeros(1023, np.float32)
+    n, inc = C.c_int(0), C.c_uint64(0)
+    N.check(N.lib().tsdrgpu_tuner_design(int(fs), float(offset_hz), float(bandwidth_hz), int(decimation), int(ntaps),
+                                         taps.ctypes.data_as(C.c_void_p), taps.size, C.byref(n), C.byref(inc)))
+    return taps[: n.value].copy(), inc.value
+
+
+def tuner_out_pairs(position: int, pairs: int, dropped: int, decimation: int) -> Tuple[int, int]:
+    """tsdrgpu_tuner_out_pairs (host only): (output pairs, output drop count) of a block."""
+    o, od = C.c_uint64(0), C.c_uint64(0)
+    N.check(N.lib().tsdrgpu_tuner_out_pairs(position, pairs, dropped, decimation, C.byref(o), C.byref(od)))
+    return o.value, od.value
+
+
+class Tuner:
+    """The digital down-converter (tsdrgpu_tuner_*): shift by offset_hz, low-pass to bandwidth_hz, decimate by D."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        h = C.c_void_p()
+        ctx.chk(ctx._lib.tsdrgpu_tuner_create(ctx._h, C.byref(h)))
+        self._h = h
+        self.config = None
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx._lib.tsdrgpu_tuner_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def configure(self, fs: int, offset_hz: float, bandwidth_hz: float, decimation: int = 1, ntaps: int = 0) -> None:
+        """Design the filter for this configuration and reset (position 0, history zero)."""
+        self.ctx.chk(self.ctx._lib.tsdrgpu_tuner_configure(self._h, int(fs), float(offset_hz), float(bandwidth_hz), int(decimation), int(ntaps)))
+        self.config = (int(fs), float(offset_hz), float(bandwidth_hz), int(decimation), int(ntaps))
+
+    @property
+    def taps(self) -> np.ndarray:
+        assert self.config is not None, "configure() first"
+        return tuner_design(*self.config)[0]
+
+    @property
+    def phase_inc(self) -> int:
+        assert self.config is not None, "configure() first"
+        return tuner_design(*self.config)[1]
+
+    def reset(self) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_tuner_reset(self._h, self.ctx.stream))
+
+    def run(self, x: torch.Tensor, dropped: int = 0) -> Tuple[torch.Tensor, int]:
+        """x: interleaved I,Q float32 on the device (the next block of the stream), preceded by `dropped` lost pairs.
+        Returns (output I,Q pairs as a float32 tensor, output drop count)."""
+        pairs = x.numel() // 2
+        D = self.config[3]
+        out = torch.empty(2 * (pairs // D + 2), dtype=torch.float32, device=self.ctx.device)
+        o, od = C.c_uint64(0), C.c_uint64(0)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_tuner_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped),
+                                                     out.data_ptr(), C.byref(o), C.byref(od)))
+        return out[: 2 * o.value], od.value
+
 
 class Resampler:
     """dsp_resample_t + dsp_resample_process (dsp.c:250-307), optionally fused with am_demod."""

@@ -26,6 +26,7 @@
 struct tsdrgpu_frd;
 struct tsdrgpu_resampler;
 struct tsdrgpu_framestage;
+struct tsdrgpu_tuner;
 
 namespace {
 
@@ -163,6 +164,10 @@ struct tsdrgpu_pipeline {
 	} sb;
 	uint32_t samplerate_real;
 	tsdrgpu_retune_cb retune_cb;
+	// tuner (tsdrgpu_pipeline_set_tuner): tn_cfg is the latest request (geo_mu), applied by the next process() call
+	struct { double offset, bw; int D, ntaps; } tn_cfg; int tn_dirty;
+	tsdrgpu_tuner *tuner; int tn_on, tn_D; uint64_t tn_pos;           // what runs; tn_pos mirrors the tuner's input position
+	float *d_tout[4]; size_t tout_cap[4];                               // the tuner's output per staging slot (floats)
 	// delivery
 	pthread_t thread; pthread_mutex_t mu; pthread_cond_t cv_job, cv_done;
 	std::deque<FrameJob> jobs; int stop; uint64_t submitted, delivered;
@@ -585,6 +590,9 @@ int tsdrgpu_pipeline_create(tsdrgpu_ctx_t *ctx, const tsdrgpu_pipeline_config_t 
 	for (int s = 0; s < 2; s++) { p->h_plot_frame[s] = NULL; p->h_plot_line[s] = NULL; p->plot_busy[s] = 0; p->h_peaks[s] = NULL; }
 	p->stop = 0; p->submitted = 0; p->delivered = 0; p->last_w = 0; p->last_h = 0;
 	memset(&p->sb, 0, sizeof p->sb); p->samplerate_real = cfg->samplerate; p->retune_cb = NULL;
+	p->tn_cfg.offset = 0; p->tn_cfg.bw = 0; p->tn_cfg.D = 1; p->tn_cfg.ntaps = 0; p->tn_dirty = 0;
+	p->tuner = NULL; p->tn_on = 0; p->tn_D = 1; p->tn_pos = 0;
+	for (int i = 0; i < 4; i++) { p->d_tout[i] = NULL; p->tout_cap[i] = 0; }
 	CU_TRY(ctx, cudaEventCreateWithFlags(&p->sb.ev, cudaEventDisableTiming));
 	memset(&p->stats, 0, sizeof p->stats);
 	CU_TRY(ctx, cudaStreamCreateWithFlags(&p->s_main, cudaStreamNonBlocking));
@@ -637,6 +645,8 @@ void tsdrgpu_pipeline_destroy(tsdrgpu_pipeline_t *p) {
 	float *dev[] = {p->d_stage[0], p->d_stage[1], p->d_stage[2], p->d_stage[3], p->d_decim, p->d_pix, p->d_frames[0], p->d_frames[1], p->d_capture[0], p->d_capture[1]};
 	for (float *d : dev) if (d) cudaFree(d);
 	for (int i = 0; i < 4; i++) if (p->d_raw[i]) cudaFree(p->d_raw[i]);
+	for (int i = 0; i < 4; i++) if (p->d_tout[i]) cudaFree(p->d_tout[i]);
+	tsdrgpu_tuner_destroy(p->tuner);
 	if (p->d_argb_last) cudaFree(p->d_argb_last);
 	for (int s = 0; s < PL_SLOTS; s++) if (p->h_frames[s]) { cudaFreeHost(p->h_frames[s]); cudaFreeHost(p->h_results[s]); cudaFreeHost(p->h_report[s]); free(p->h_pll_rr[s]); }
 	cudaEventDestroy(p->ev_res);
@@ -666,8 +676,25 @@ int tsdrgpu_pipeline_set_resolution(tsdrgpu_pipeline_t *p, int height, double re
 int tsdrgpu_pipeline_set_samplerate(tsdrgpu_pipeline_t *p, uint32_t samplerate) {
 	if (!p || samplerate == 0) return TSDRGPU_EINVAL;
 	pthread_mutex_lock(&p->geo_mu);
-	p->samplerate = samplerate; p->samplerate_real = samplerate;
+	if (p->tn_cfg.bw > 0) {                              // tuned: the taps are re-designed for the new rate (next process() call)
+		const int rc = tsdrgpu_tuner_design(samplerate, p->tn_cfg.offset, p->tn_cfg.bw, p->tn_cfg.D, p->tn_cfg.ntaps, NULL, 0, NULL, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+		p->tn_dirty = 1;
+	}
+	p->samplerate = p->tn_cfg.bw > 0 ? samplerate / (uint32_t) p->tn_cfg.D : samplerate; p->samplerate_real = samplerate;
 	geometry_locked(p);
+	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_set_tuner(tsdrgpu_pipeline_t *p, double offset_hz, double bandwidth_hz, int decimation, int ntaps) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	pthread_mutex_lock(&p->geo_mu);
+	if (bandwidth_hz > 0) {
+		const int rc = tsdrgpu_tuner_design(p->samplerate_real, offset_hz, bandwidth_hz, decimation, ntaps, NULL, 0, NULL, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+	}
+	p->tn_cfg.offset = offset_hz; p->tn_cfg.bw = bandwidth_hz > 0 ? bandwidth_hz : 0; p->tn_cfg.D = bandwidth_hz > 0 ? decimation : 1; p->tn_cfg.ntaps = ntaps;
+	p->tn_dirty = 1;
 	pthread_mutex_unlock(&p->geo_mu);
 	return TSDRGPU_OK;
 }
@@ -727,9 +754,42 @@ static void superb_stop(tsdrgpu_pipeline *p) {                  // superbandwidt
 	p->sb.state = SB_STOPPED;
 	if (p->retune_cb) p->retune_cb(0, p->user);
 	pthread_mutex_lock(&p->geo_mu);
-	p->samplerate = p->samplerate_real;
+	p->samplerate = p->samplerate_real / (uint32_t) p->tn_D;
 	geometry_locked(p);
 	pthread_mutex_unlock(&p->geo_mu);
+	if (p->tn_on) { p->tn_pos = 0; tsdrgpu_tuner_reset(p->tuner, p->s_ingest); }     // the tuner resumes from a clean start
+}
+
+// a tuner (re)configuration, at the start of a process() call: the stream starts over at the new internal rate
+static int tuner_apply(tsdrgpu_pipeline *p) {
+	tsdrgpu_ctx_t *ctx = p->ctx;
+	int rc;
+	pthread_mutex_lock(&p->geo_mu);
+	const int dirty = p->tn_dirty; const double offset = p->tn_cfg.offset, bw = p->tn_cfg.bw; const int D = p->tn_cfg.D, ntaps = p->tn_cfg.ntaps;
+	const uint32_t fs = p->samplerate_real;
+	p->tn_dirty = 0;
+	pthread_mutex_unlock(&p->geo_mu);
+	if (!dirty) return TSDRGPU_OK;
+	if ((rc = tsdrgpu_framestage_join(p->fs, p->s_main))) return rc;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_copy)); CU_TRY(ctx, cudaStreamSynchronize(p->s_ingest));
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_main)); CU_TRY(ctx, cudaStreamSynchronize(p->s_out));
+	if (bw > 0) {
+		if (!p->tuner && (rc = tsdrgpu_tuner_create(ctx, &p->tuner))) return rc;
+		if ((rc = tsdrgpu_tuner_configure(p->tuner, fs, offset, bw, D, ntaps))) return rc;
+		p->tn_on = 1; p->tn_D = D;
+	} else { p->tn_on = 0; p->tn_D = 1; }
+	p->tn_pos = 0;
+	// what waits at the old rate is meaningless at the new one: start over behind the tuner as a new pipeline would
+	p->decim_fill = 0; p->decim_read = 0; p->decim_elem = 2; p->pix_fill = 0; p->pix_read = 0; p->cap_fill = 0;
+	p->dev_drop = DropComp(); p->pix_drop = DropComp();
+	if ((rc = tsdrgpu_resampler_reset(p->rs, p->s_main))) return rc;
+	if ((rc = tsdrgpu_framestage_reset(p->fs, p->s_main))) return rc;
+	if ((rc = tsdrgpu_frd_reset(p->frd))) return rc;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_main));
+	pthread_mutex_lock(&p->geo_mu);
+	if (p->sb.state == SB_STOPPED) { p->samplerate = p->samplerate_real / (uint32_t) p->tn_D; geometry_locked(p); }
+	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
 }
 // make room for `bytes` of raw samples in slot ss (contents are not preserved)
 static int raw_reserve(tsdrgpu_pipeline *p, int ss, size_t bytes) {
@@ -933,6 +993,8 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	ARG_TRY(ctx, fmt >= TSDRGPU_FMT_FLOAT && fmt <= TSDRGPU_FMT_UINT16);
 	ARG_TRY(ctx, (items_count & 1) == 0);                     // assert at TSDRLibrary.c:265
 	const uint64_t size2 = items_count >> 1;
+	int rc = tuner_apply(p);
+	if (rc) return rc;
 	pthread_mutex_lock(&p->geo_mu);
 	const int w = p->width, h = p->height; const double ptos = p->ptos;
 	pthread_mutex_unlock(&p->geo_mu);
@@ -942,18 +1004,28 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	superb_stop(p);
 	const int block = (int) round((double) ((w * h) << 1) * ptos);           // TSDRLibrary.c:284
 	if (block <= 0) return TSDRGPU_OK;
-	p->dev_drop.shift_with((uint32_t) block, samples_dropped);
-	const bool drop_all = p->dev_drop.will_drop_all((uint32_t) size2);
+	// what the stages behind the tuner see: its output pairs and output drop count (the block itself when there is no tuner)
+	const bool tuned = p->tn_on != 0;
+	const uint64_t gap = samples_dropped > 0 ? (uint64_t) samples_dropped : 0;
+	uint64_t n2 = size2; int64_t dropped = samples_dropped;
+	if (tuned) {
+		uint64_t o = 0, od = 0;
+		tsdrgpu_tuner_out_pairs(p->tn_pos, size2, gap, p->tn_D, &o, &od);
+		n2 = o; dropped = (int64_t) od;
+	}
+	p->dev_drop.shift_with((uint32_t) block, dropped);
+	const bool drop_all = p->dev_drop.will_drop_all((uint32_t) n2);
 	const bool plots_on = !p->params[TSDRGPU_PARAM_AUTOCORR_PLOTS_OFF];
-	int rc = TSDRGPU_OK;
-	const bool need_data = size2 > 0 && (!drop_all || (plots_on && samples_dropped != 0));
+	const bool need_data = n2 > 0 && (!drop_all || (plots_on && dropped != 0));
+	// the tuner sees every non-empty block, also one the drop compensation discards whole: its history and position stay continuous
+	const bool need_copy = tuned ? size2 > 0 : need_data;
 	const int ss = p->stage_slot;
-	float *stage = NULL;
+	float *stage = NULL, *d_in = NULL;
 	bool copy_issued = false;
 	// Every path out of this block -- success or failure -- passes the synchronisation of the copy stream below: the header's
 	// contract is that the caller's buffer is read during the call only.
 	do {
-		if (need_data) {
+		if (need_copy) {
 			if (h_iq == NULL) { rc = tsdrgpu_fail(ctx, TSDRGPU_EINVAL, "invalid argument: h_iq != NULL", cudaSuccess, __FILE__, __LINE__); break; }
 			p->stage_slot = (p->stage_slot + 1) & 3;
 			if (p->stage_cap[ss] < items_count) { cudaStreamSynchronize(p->s_ingest); cudaStreamSynchronize(p->s_copy); }
@@ -978,10 +1050,25 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 				if ((e = cudaGetLastError()) != cudaSuccess) { rc = tsdrgpu_fail(ctx, TSDRGPU_ECUDA, "kernel launch", e, __FILE__, __LINE__); break; }
 			}
 			p->stats.h2d_bytes += bytes;
-			if ((rc = feed_capture(p, stage, size2, samples_dropped != 0))) break;
-		} else if (plots_on && samples_dropped != 0) p->cap_fill = 0;
+			d_in = stage;
+			if (tuned) {                                                       // shift, low-pass, decimate (tuner.cu)
+				if (p->tout_cap[ss] < 2 * n2 + 2) cudaStreamSynchronize(p->s_ingest);
+				if ((rc = grow(ctx, p->s_ingest, &p->d_tout[ss], &p->tout_cap[ss], 2 * n2 + 2, 0))) break;
+				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, stage, size2, gap, p->d_tout[ss], NULL, NULL))) break;
+				p->tn_pos += gap + size2;
+				d_in = p->d_tout[ss];
+			}
+			if (need_data) { if ((rc = feed_capture(p, d_in, n2, dropped != 0))) break; }
+			else if (plots_on && dropped != 0) p->cap_fill = 0;
+		} else {
+			if (tuned && gap > 0) {                                            // an empty block that only reports a loss
+				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, NULL, 0, gap, NULL, NULL, NULL))) break;
+				p->tn_pos += gap;
+			}
+			if (plots_on && dropped != 0) p->cap_fill = 0;
+		}
 		uint32_t skip = 0;
-		const uint32_t fwd = p->dev_drop.add((uint32_t) size2, (uint32_t) block, true, &skip);
+		const uint32_t fwd = p->dev_drop.add((uint32_t) n2, (uint32_t) block, true, &skip);
 		if (fwd) {
 			float *where;
 			if ((rc = decim_set_elem(p, 2))) break;
@@ -989,7 +1076,7 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 			if ((rc = decim_reserve(p, fwd, &where))) break;
 			cudaError_t e = cudaStreamWaitEvent(p->s_ingest, p->ev_decim, 0);  // the last compaction of the decimator input is done
 			if (e == cudaSuccess) {
-				pl_copy_f32<<<(unsigned) ((2ull * fwd + 255) / 256 < 2048 ? (2ull * fwd + 255) / 256 : 2048), 256, 0, p->s_ingest>>>(stage + 2ull * skip, where, 2ull * fwd);
+				pl_copy_f32<<<(unsigned) ((2ull * fwd + 255) / 256 < 2048 ? (2ull * fwd + 255) / 256 : 2048), 256, 0, p->s_ingest>>>(d_in + 2ull * skip, where, 2ull * fwd);
 				ctx->launches++;
 				e = cudaGetLastError();
 			}
@@ -998,7 +1085,7 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 		}
 		{
 			cudaError_t e = cudaSuccess;
-			if (need_data) e = cudaEventRecord(p->ev_used[ss], p->s_ingest);  // the slot may be overwritten after this point
+			if (need_copy) e = cudaEventRecord(p->ev_used[ss], p->s_ingest);  // the slot may be overwritten after this point
 			if (e == cudaSuccess) e = cudaEventRecord(p->ev_ingest, p->s_ingest);
 			if (e == cudaSuccess) e = cudaStreamWaitEvent(p->s_main, p->ev_ingest, 0);      // the resampler may read what was appended
 			if (e != cudaSuccess) { rc = tsdrgpu_fail(ctx, TSDRGPU_ECUDA, "stream ordering", e, __FILE__, __LINE__); break; }

@@ -67,6 +67,9 @@ struct tsdr_lib {
 	/* optional timing of the data callback (TSDR_STATS_FILE=<path>): where a run's wall time goes, per block */
 	int stats_on; uint64_t cb_count; double cb_inside_s, cb_outside_s, cb_last_exit;
 	struct { double t, inside, outside; uint64_t n; } cb_log[1024]; int cb_nlog;   /* cumulative values every 128 callbacks (CLOCK_MONOTONIC) */
+	/* TSDR_TUNER=<offset_hz>,<bandwidth_hz>[,<decimation>[,<ntaps>]] (read by tsdr_readasync): the run demodulates that sub-band
+	 * only, at samplerate_real / tuner_d (1 = no tuner) */
+	double tn_offset, tn_bw; int tuner_d, tn_ntaps;
 };
 
 /* ---- error text: library-owned, NULL after a successful call (TSDRLibrary.c:136-159) ---------------------- */
@@ -159,8 +162,30 @@ int tsdr_getsamplerate(tsdr_lib_t *t) {
 	if (!t->plugin.initialized) return fail(t, "Cannot change sample rate. Plugin not loaded yet.", TSDR_ERR_PLUGIN);
 	t->samplerate_real = t->plugin.getsamplerate();
 	if (t->samplerate_real == 0 || t->samplerate_real > MAX_SAMPLE_RATE) return fail(t, "Invalid/unsupported value for sample rate.", TSDR_SAMPLE_RATE_WRONG);
-	set_internal_samplerate(t, t->samplerate_real);
+	set_internal_samplerate(t, t->samplerate_real / (uint32_t) (t->tuner_d > 1 ? t->tuner_d : 1));
 	return ok(t);
+}
+
+/* TSDR_TUNER: numbers separated by commas, all of them consumed; checked against the plugin's rate by the tuner's own rules */
+static int parse_tuner(tsdr_lib_t *t, const char *text) {
+	double v[4] = {0.0, 0.0, 1.0, 0.0};
+	int n = 0;
+	const char *c = text;
+	for (;;) {
+		char *e;
+		const double x = strtod(c, &e);
+		if (e == c || n == 4) { n = -1; break; }
+		v[n++] = x; c = e;
+		while (*c == ' ') c++;
+		if (*c != ',') break;
+		c++;
+	}
+	if (n < 2 || *c != '\0' || !(v[2] >= 1.0 && v[2] <= 1024.0 && v[2] == (double) (int) v[2]) || !(v[3] >= 0.0 && v[3] <= 65536.0 && v[3] == (double) (int) v[3]))
+		return fail(t, "TSDR_TUNER: expected <offset_hz>,<bandwidth_hz>[,<decimation>[,<ntaps>]] with an integer decimation and ntaps", TSDR_INVALID_PARAMETER_VALUE);
+	if (tsdrgpu_tuner_design(t->samplerate_real, v[0], v[1], (int) v[2], (int) v[3], NULL, 0, NULL, NULL) != TSDRGPU_OK)
+		return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
+	t->tn_offset = v[0]; t->tn_bw = v[1]; t->tuner_d = (int) v[2]; t->tn_ntaps = (int) v[3];
+	return TSDR_OK;
 }
 
 int tsdr_setbasefreq(tsdr_lib_t *t, uint32_t freq) {
@@ -333,7 +358,15 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	tsdr_reset(t);
 	t->nativerunning = 1; t->running = 1; t->gpu_failed = 0;
 	int status, pluginsfault = 0;
+	t->tuner_d = 1; t->tn_bw = 0.0;
 	if ((status = tsdr_getsamplerate(t)) != TSDR_OK) goto end;
+	{
+		const char *tuner = getenv("TSDR_TUNER");
+		if (tuner && tuner[0]) {
+			if ((status = parse_tuner(t, tuner)) != TSDR_OK) goto end;
+			set_internal_samplerate(t, t->samplerate_real / (uint32_t) t->tuner_d);     /* the geometry of the tuned sub-band */
+		}
+	}
 	if (t->width <= 0 || t->height <= 0 || (long long) t->width * t->height > MAX_PIXELS) {
 		status = fail(t, "The supplied height and the width are invalid!", TSDR_WRONG_VIDEOPARAMS);
 		goto end;
@@ -364,7 +397,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	{
 		tsdrgpu_pipeline_config_t cfg;
 		memset(&cfg, 0, sizeof cfg);
-		cfg.samplerate = t->samplerate; cfg.height = t->height; cfg.refreshrate = t->refreshrate; cfg.motionblur = t->motionblur;
+		cfg.samplerate = t->samplerate_real; cfg.height = t->height; cfg.refreshrate = t->refreshrate; cfg.motionblur = t->motionblur;
 		memcpy(cfg.params_int, t->params_int, sizeof cfg.params_int);
 		const char *bf = getenv("TSDR_BATCH_FRAMES");
 		cfg.batch_frames = bf ? atoi(bf) : 1;               /* 1 frame per launch: lowest latency for an interactive host */
@@ -379,6 +412,11 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 		tsdrgpu_pipeline_set_retune(np, on_retune);
 		/* a plugin keeps its buffer for the whole tsdrplugin_readasync (TSDRPlugin_RawFile.c:212, 263): page-lock it in place */
 		tsdrgpu_pipeline_set_host_registration(np, getenv("TSDR_NO_HOST_REGISTER") ? 0 : 1);
+		if (t->tn_bw > 0 && tsdrgpu_pipeline_set_tuner(np, t->tn_offset, t->tn_bw, t->tuner_d, t->tn_ntaps) != TSDRGPU_OK) {
+			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_INVALID_PARAMETER_VALUE);
+			tsdrgpu_pipeline_destroy(np);
+			goto end;
+		}
 		if (ndev > 1 && tsdrgpu_pipeline_set_superb_devices(np, devlist, ndev) != TSDRGPU_OK) {
 			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_CANNOT_OPEN_DEVICE);
 			tsdrgpu_pipeline_destroy(np);
@@ -418,6 +456,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	}
 	if (t->gpu_failed) status = TSDR_CANNOT_OPEN_DEVICE;
 end:
+	t->tuner_d = 1;
 	if (pluginsfault) fail(t, t->plugin.getlasterrortext(), status);
 	pthread_mutex_lock(&t->mu);
 	t->running = 0; t->nativerunning = 0;

@@ -115,6 +115,14 @@ class Pipeline:
     def set_resolution(self, height: int, refreshrate: float) -> None:
         N.check(self._lib.tsdrgpu_pipeline_set_resolution(self._h, height, refreshrate), self._ctx)
 
+    def set_tuner(self, offset_hz: float, bandwidth_hz: float, decimation: int = 1, ntaps: int = 0) -> None:
+        """Demodulate only the sub-band of `bandwidth_hz` around `offset_hz`, decimated by `decimation` (the pipeline then runs
+        at samplerate / decimation); bandwidth_hz <= 0 switches the tuner off.  Takes effect at the next process() call."""
+        N.check(self._lib.tsdrgpu_pipeline_set_tuner(self._h, float(offset_hz), float(bandwidth_hz), int(decimation), int(ntaps)), self._ctx)
+
+    def set_samplerate(self, samplerate: int) -> None:
+        N.check(self._lib.tsdrgpu_pipeline_set_samplerate(self._h, int(samplerate)), self._ctx)
+
     def set_superb_devices(self, devices) -> None:
         """Superbandwidth mode with one hop per GPU: devices[0] is this pipeline's device, len(devices) in {2, 4, 8} = hops."""
         arr = (C.c_int * len(devices))(*devices)
