@@ -362,6 +362,60 @@ TSDRGPU_API int  tsdrgpu_tuner_reset(tsdrgpu_tuner_t *t, void *stream);      /* 
 TSDRGPU_API int  tsdrgpu_tuner_run(tsdrgpu_tuner_t *t, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before, float *d_out,
                                    uint64_t *out_pairs, uint64_t *out_dropped);
 
+/* ---------------------------------------------------------------------------- channelizer (polyphase filter bank)
+ * Not in the reference: splits a capture into K sub-bands at once (DESIGN.md section 5.7).  K is a power of two in 2..256, the
+ * decimation is D = K/2 (oversampled by 2), Q taps per channel in 4..32 (0 = 16).  The prototype h is the tuner's design
+ * tsdrgpu_tuner_design(fs, 0, fs / K, K / 2, Q * K - 1).  Channel c has offset c * fs / K for c < K/2 and (c - K) * fs / K otherwise
+ * (channel K/2 reads -fs/2) and output
+ *   y_c[m] = sum_k h[k] x[mD - k] e^{-2 pi i off_c (mD - k) / fs},
+ * x with zeros before the stream and over every drop, n counted since the last reset: the tuner at off_c with the same taps and
+ * decimation.  Output m exists for every mD inside a block, so the counts are tsdrgpu_channelizer_out_pairs's.
+ * Configuration rules: K a power of two in 2..256, Q in 4..32 (0 = default), fs % (K/2) == 0, 2 fs / K >= 130500 (the channel
+ * rate keeps the frame-rate detector's line window off lag 0), Q*K - 1 taps fit the shared-memory tile; anything else is
+ * TSDRGPU_EINVAL with a text naming the rule. */
+typedef struct tsdrgpu_channelizer tsdrgpu_channelizer_t;
+enum { TSDRGPU_CHANNELIZER_COMPLEX = 0, TSDRGPU_CHANNELIZER_MAGNITUDE = 1 };
+/* host-only: validates and returns the Q*K - 1 float32 prototype taps (taps may be NULL: validation only) */
+TSDRGPU_API int tsdrgpu_channelizer_design(uint32_t fs, int channels, int taps_per_channel, float *taps, int cap, int *ntaps_out);
+/* host-only: the tuner's count arithmetic (tsdrgpu_tuner_out_pairs) at D = channels / 2, outputs per channel */
+TSDRGPU_API int tsdrgpu_channelizer_out_pairs(uint64_t position, uint64_t pairs, uint64_t dropped, int channels, uint64_t *out_pairs,
+                                              uint64_t *out_dropped);
+TSDRGPU_API int  tsdrgpu_channelizer_create(tsdrgpu_ctx_t *ctx, tsdrgpu_channelizer_t **c);
+TSDRGPU_API void tsdrgpu_channelizer_destroy(tsdrgpu_channelizer_t *c);
+TSDRGPU_API int  tsdrgpu_channelizer_configure(tsdrgpu_channelizer_t *c, uint32_t fs, int channels, int taps_per_channel);   /* synchronises */
+TSDRGPU_API int  tsdrgpu_channelizer_reset(tsdrgpu_channelizer_t *c, void *stream);       /* position 0, history zero */
+/* mode TSDRGPU_CHANNELIZER_COMPLEX: channel c's *out_pairs I,Q pairs at d_out + 2 * c * channel_stride floats;
+ * TSDRGPU_CHANNELIZER_MAGNITUDE: sqrtf(I*I + Q*Q) (tsdrgpu_am_demod's arithmetic) at d_out + c * channel_stride floats.
+ * channel_stride (in outputs) >= *out_pairs.  Asynchronous; the history of the last Q*K - 2 input pairs is carried on the device. */
+TSDRGPU_API int  tsdrgpu_channelizer_run(tsdrgpu_channelizer_t *c, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before,
+                                         int mode, float *d_out, uint64_t channel_stride, uint64_t *out_pairs, uint64_t *out_dropped);
+
+/* ---------------------------------------------------------------------------- scan (a frame-rate detector per channel)
+ * A channelizer in magnitude mode; each channel's stream is cut into consecutive captures of tsdrgpu_frd_capture_size(rate)
+ * samples, rate = 2 fs / K (a drop discards every channel's partial capture).  Every complete round of K captures goes through the
+ * batched autocorrelation and updates K pairs of running means over tsdrgpu_frd_windows(rate), on an internal stream behind the
+ * caller's.  Per channel the table reports the first strict maximum of each plot, the video mode they imply
+ * (tsdrgpu_videomode_from_peaks) and score = (max - mean) / std of each plot. */
+typedef struct {
+	double   offset_hz;                  /* the channel's centre, in the frame of tsdrgpu_pipeline_set_tuner's offset_hz */
+	uint32_t rate;                       /* 2 fs / K */
+	uint64_t captures;                   /* rounds accumulated since the last reset */
+	int32_t  frame_index, line_index;    /* first strict maximum of each plot (indices into the windows) */
+	double   fps; int32_t height;        /* tsdrgpu_videomode_from_peaks at `rate` (0 before the first round) */
+	double   frame_score, line_score;
+} tsdrgpu_scan_channel_t;
+typedef struct tsdrgpu_scan tsdrgpu_scan_t;
+TSDRGPU_API int  tsdrgpu_scan_create(tsdrgpu_ctx_t *ctx, tsdrgpu_scan_t **s);
+TSDRGPU_API void tsdrgpu_scan_destroy(tsdrgpu_scan_t *s);
+TSDRGPU_API int  tsdrgpu_scan_configure(tsdrgpu_scan_t *s, uint32_t fs, int channels, int taps_per_channel);            /* synchronises */
+TSDRGPU_API int  tsdrgpu_scan_reset(tsdrgpu_scan_t *s, void *stream);
+TSDRGPU_API int  tsdrgpu_scan_run(tsdrgpu_scan_t *s, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before);
+/* min(cap, K) records, channel order; synchronises */
+TSDRGPU_API int  tsdrgpu_scan_results(tsdrgpu_scan_t *s, void *stream, tsdrgpu_scan_channel_t *h_out, int cap);
+/* the running means, channel-major: channel c's frame plot at h_plots[c * (frame_len + line_len)], its line plot right behind;
+ * synchronises */
+TSDRGPU_API int  tsdrgpu_scan_plots(tsdrgpu_scan_t *s, void *stream, double *h_plots, uint64_t cap, int *frame_len, int *line_len);
+
 /* ---------------------------------------------------------------------------- a1, a3, a5, a16, a17  streaming pipeline
  * replaces the body of process() (TSDRLibrary.c:264-298), decimatingthread / postprocessingthread /
  * videodecodingthread (TSDRLibrary.c:300-418) with their three rings (circbuff.c), dsp_dropped_compensation_*
@@ -429,6 +483,13 @@ TSDRGPU_API int  tsdrgpu_pipeline_set_samplerate(tsdrgpu_pipeline_t *p, uint32_t
  * and frame-rate detector reset.  Superbandwidth mode bypasses the tuner and resumes it, reset, when it ends.
  * set_samplerate re-designs the taps for the new rate and rejects a rate the current tuning cannot take. */
 TSDRGPU_API int  tsdrgpu_pipeline_set_tuner(tsdrgpu_pipeline_t *p, double offset_hz, double bandwidth_hz, int decimation, int ntaps);
+/* The scan (see tsdrgpu_scan_*) over the wideband blocks: every non-empty block after it reaches the device, ahead of the tuner, so
+ * its offsets are in the tuner's frame.  channels = 0 switches it off (the default).  Checked against the current rate at once;
+ * takes effect, reset, at the next process() call.  It changes nothing the pixel path produces; its heavy part runs on a stream of
+ * its own.  Superbandwidth mode pauses it; it resumes, reset, when that mode ends.  set_samplerate re-validates it. */
+TSDRGPU_API int  tsdrgpu_pipeline_set_scan(tsdrgpu_pipeline_t *p, int channels, int taps_per_channel);
+/* the scan's table (tsdrgpu_scan_results): *n = records written (0 while no scan runs); synchronises */
+TSDRGPU_API int  tsdrgpu_pipeline_scan_results(tsdrgpu_pipeline_t *p, tsdrgpu_scan_channel_t *out, int cap, int *n);
 /* superbandwidth mode (PARAM_AUTOCORR_SUPERRESOLUTION = 1; superb_run, superbandwidth.c:179-254) retunes the front end
  * between hops through this callback; without it the hops are recorded at one frequency */
 TSDRGPU_API int  tsdrgpu_pipeline_set_retune(tsdrgpu_pipeline_t *p, tsdrgpu_retune_cb cb);

@@ -35,6 +35,13 @@ class PipelineStats(C.Structure):
                                           "h2d_bytes", "d2h_bytes", "gpu_launches", "stitches", "host_buffers_registered")]
 
 
+class ScanChannel(C.Structure):
+    """tsdrgpu_scan_channel_t"""
+    _fields_ = [("offset_hz", C.c_double), ("rate", C.c_uint32), ("captures", C.c_uint64), ("frame_index", C.c_int32),
+                ("line_index", C.c_int32), ("fps", C.c_double), ("height", C.c_int32), ("frame_score", C.c_double),
+                ("line_score", C.c_double)]
+
+
 FRAME_CB = C.CFUNCTYPE(None, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_void_p)
 VALUE_CB = C.CFUNCTYPE(None, C.c_int, C.c_double, C.c_double, C.c_void_p)
 PLOT_CB = C.CFUNCTYPE(None, C.c_int, C.c_int, C.POINTER(C.c_double), C.c_int, C.c_uint32, C.c_void_p)
@@ -157,6 +164,23 @@ _SIGS = {
     "tsdrgpu_tuner_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
     "tsdrgpu_tuner_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
                                     C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_channelizer_design": (C.c_int, [C.c_uint32, C.c_int, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int)]),
+    "tsdrgpu_channelizer_out_pairs": (C.c_int, [C.c_uint64, C.c_uint64, C.c_uint64, C.c_int, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_channelizer_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "tsdrgpu_channelizer_destroy": (None, [C.c_void_p]),
+    "tsdrgpu_channelizer_configure": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_int]),
+    "tsdrgpu_channelizer_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tsdrgpu_channelizer_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int, C.c_void_p, C.c_uint64,
+                                          C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_scan_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "tsdrgpu_scan_destroy": (None, [C.c_void_p]),
+    "tsdrgpu_scan_configure": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_int]),
+    "tsdrgpu_scan_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tsdrgpu_scan_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]),
+    "tsdrgpu_scan_results": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(ScanChannel), C.c_int]),
+    "tsdrgpu_scan_plots": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "tsdrgpu_pipeline_set_scan": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
+    "tsdrgpu_pipeline_scan_results": (C.c_int, [C.c_void_p, C.POINTER(ScanChannel), C.c_int, C.POINTER(C.c_int)]),
     "tsdrgpu_pipeline_set_retune": (C.c_int, [C.c_void_p, RETUNE_CB]),
     "tsdrgpu_pipeline_set_motionblur": (C.c_int, [C.c_void_p, C.c_float]),
     "tsdrgpu_pipeline_set_host_registration": (C.c_int, [C.c_void_p, C.c_int]),

@@ -186,6 +186,12 @@ class Context:
     def tuner(self) -> "Tuner":
         return Tuner(self)
 
+    def channelizer(self) -> "Channelizer":
+        return Channelizer(self)
+
+    def scan(self) -> "Scan":
+        return Scan(self)
+
 
 def tuner_design(fs: int, offset_hz: float, bandwidth_hz: float, decimation: int = 1, ntaps: int = 0) -> Tuple[np.ndarray, int]:
     """tsdrgpu_tuner_design (host only): the float32 taps and the 64-bit phase increment round(offset / fs * 2^64) (as an
@@ -250,6 +256,125 @@ class Tuner:
         self.ctx.chk(self.ctx._lib.tsdrgpu_tuner_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped),
                                                      out.data_ptr(), C.byref(o), C.byref(od)))
         return out[: 2 * o.value], od.value
+
+
+def channelizer_design(fs: int, channels: int, taps_per_channel: int = 0) -> np.ndarray:
+    """tsdrgpu_channelizer_design (host only): the float32 prototype taps (Q*K - 1 of them).  Raises TsdrGpuError naming the
+    violated rule."""
+    taps = np.zeros(32 * 256, np.float32)
+    n = C.c_int(0)
+    N.check(N.lib().tsdrgpu_channelizer_design(int(fs), int(channels), int(taps_per_channel), taps.ctypes.data_as(C.c_void_p), taps.size,
+                                               C.byref(n)))
+    return taps[: n.value].copy()
+
+
+def channelizer_out_pairs(position: int, pairs: int, dropped: int, channels: int) -> Tuple[int, int]:
+    """tsdrgpu_channelizer_out_pairs (host only): (outputs per channel, output drop count) of a block."""
+    o, od = C.c_uint64(0), C.c_uint64(0)
+    N.check(N.lib().tsdrgpu_channelizer_out_pairs(position, pairs, dropped, channels, C.byref(o), C.byref(od)))
+    return o.value, od.value
+
+
+def channel_offsets(fs: int, channels: int) -> np.ndarray:
+    """Centre of every channel in Hz: c fs / K for c < K/2, (c - K) fs / K otherwise."""
+    c = np.arange(channels)
+    return np.where(c < channels // 2, c, c - channels) * (fs / channels)
+
+
+class Channelizer:
+    """The polyphase filter bank (tsdrgpu_channelizer_*): K channels at offsets c fs / K, each decimated by K/2."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        h = C.c_void_p()
+        ctx.chk(ctx._lib.tsdrgpu_channelizer_create(ctx._h, C.byref(h)))
+        self._h = h
+        self.config = None
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx._lib.tsdrgpu_channelizer_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def configure(self, fs: int, channels: int, taps_per_channel: int = 0) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_channelizer_configure(self._h, int(fs), int(channels), int(taps_per_channel)))
+        self.config = (int(fs), int(channels), int(taps_per_channel))
+
+    def reset(self) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_channelizer_reset(self._h, self.ctx.stream))
+
+    def run(self, x: torch.Tensor, dropped: int = 0, magnitude: bool = False) -> Tuple[torch.Tensor, int]:
+        """x: interleaved I,Q float32 on the device, preceded by `dropped` lost pairs.  Returns (outputs, output drop count): a
+        [K, M, 2] float32 tensor of I,Q pairs, or [K, M] magnitudes."""
+        pairs = x.numel() // 2
+        K = self.config[1]
+        stride = pairs // (K // 2) + 2
+        out = torch.empty((K, stride, 1 if magnitude else 2), dtype=torch.float32, device=self.ctx.device)
+        o, od = C.c_uint64(0), C.c_uint64(0)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_channelizer_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped),
+                                                           int(magnitude), out.data_ptr(), stride, C.byref(o), C.byref(od)))
+        out = out[:, : o.value]
+        return (out[..., 0] if magnitude else out), od.value
+
+
+def scan_table(records, n: int):
+    """tsdrgpu_scan_channel_t records -> list of dicts (with the channel number), sorted by frame_score, highest first."""
+    rows = []
+    for c in range(n):
+        r = records[c]
+        rows.append({"channel": c, **{f: getattr(r, f) for f, _ in N.ScanChannel._fields_}})
+    return sorted(rows, key=lambda d: -d["frame_score"])
+
+
+class Scan:
+    """A frame-rate detector on every channel of a channelizer (tsdrgpu_scan_*): which sub-bands hold a raster, in which mode."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        h = C.c_void_p()
+        ctx.chk(ctx._lib.tsdrgpu_scan_create(ctx._h, C.byref(h)))
+        self._h = h
+        self.channels = 0
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx._lib.tsdrgpu_scan_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def configure(self, fs: int, channels: int, taps_per_channel: int = 0) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_configure(self._h, int(fs), int(channels), int(taps_per_channel)))
+        self.channels = int(channels)
+
+    def reset(self) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_reset(self._h, self.ctx.stream))
+
+    def run(self, x: torch.Tensor, dropped: int = 0) -> None:
+        pairs = x.numel() // 2
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped)))
+
+    def records(self):
+        """The raw table, channel order (ScanChannel structures)."""
+        recs = (N.ScanChannel * self.channels)()
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_results(self._h, self.ctx.stream, recs, self.channels))
+        return recs
+
+    def results(self):
+        """One dict per channel, sorted by frame_score, highest first."""
+        return scan_table(self.records(), self.channels)
+
+    def plots(self) -> Tuple[np.ndarray, int, int]:
+        """The running means, [K, frame_len + line_len] float64, and the two window lengths."""
+        fl, ll = C.c_int(0), C.c_int(0)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_plots(self._h, self.ctx.stream, None, 0, C.byref(fl), C.byref(ll)))
+        out = np.zeros((self.channels, fl.value + ll.value), np.float64)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_scan_plots(self._h, self.ctx.stream, out.ctypes.data_as(C.c_void_p), out.size, None, None))
+        return out, fl.value, ll.value
 
 
 class Resampler:

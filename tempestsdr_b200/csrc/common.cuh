@@ -92,3 +92,10 @@ int tsdrgpu_fft_batch_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const fl
                                float2 *scratch, unsigned long long n_pow2, unsigned batch, int inverse);
 int tsdrgpu_ifft_abs_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, float2 *data, float *real_out, unsigned long long n_pow2);
 int tsdrgpu_argmax_mag_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const float2 *x, unsigned n, void *d_part, int *d_result);
+// the tuner's filter designer (tuner.cu), shared with the channelizer: n float32 taps of a Kaiser-windowed sinc low-pass
+void tsdrgpu_kaiser_lowpass_internal(uint32_t fs, double bandwidth_hz, int n, float *taps);
+// the scan's per-plot result (fft.cu's k_plot_scores): first strict maximum and (max - mean) / std
+struct TsdrScanPeak { double score; int32_t index, pad; };
+int tsdrgpu_scan_round_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const float *d_caps, uint64_t cap_stride, uint32_t size,
+                                unsigned K, uint32_t rate, float *d_big, float2 *w0, float2 *w1, double *d_plots, uint64_t calls,
+                                TsdrScanPeak *d_res);

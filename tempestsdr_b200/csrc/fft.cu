@@ -528,6 +528,54 @@ __global__ void __launch_bounds__(1024) k_plot_peaks(const double *p0, int n0, c
 		peaks[blockIdx.x] = (n <= 0 || first != first || bi == 0x7fffffff) ? 0 : bi;
 	}
 }
+// the scan (channelizer.cu): the running means of K channels at once, one capture each.  Channel y's answer starts at
+// in + y * in_stride, its plots at out + y * out_stride ([frame window | line window]); the same arithmetic as k_accumulate_batch
+// with batch = 1.
+__global__ void k_accumulate_channels(double *out, long long out_stride, unsigned long long calls, const float2 *in, long long in_stride,
+                                      int fmin, int flen, int lmin, int llen) {
+	double *o = out + (long long) blockIdx.y * out_stride;
+	const float2 *a = in + (long long) blockIdx.y * in_stride;
+	for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < flen + llen; i += gridDim.x * blockDim.x) {
+		const float2 v = a[i < flen ? fmin + i : lmin + (i - flen)];
+		const double re = (double) v.x, im = (double) v.y;
+		const double mag = __dsqrt_rn(__dadd_rn(__dmul_rn(re, re), __dmul_rn(im, im)));
+		o[i] = (calls == 0) ? mag : __ddiv_rn(__dadd_rn(__dmul_rn(o[i], (double) (calls - 1)), mag), (double) calls);
+	}
+}
+// One CTA per plot of every channel (CTA b: channel b / 2, frame plot for even b, line plot for odd b): the first strict maximum
+// with k_plot_peaks's rule, and score = (max - mean) / std over the plot (population std; 0 when std is 0), sums in double.
+__global__ void __launch_bounds__(1024) k_plot_scores(const double *plots, long long stride, int flen, int llen, TsdrScanPeak *res) {
+	__shared__ double s_v[32], s_s[32], s_q[32]; __shared__ int s_i[32];
+	const double *v = plots + (long long) (blockIdx.x >> 1) * stride + ((blockIdx.x & 1) ? flen : 0);
+	const int n = (blockIdx.x & 1) ? llen : flen;
+	double best = -INFINITY, sum = 0.0, sq = 0.0; int bi = 0x7fffffff;
+	for (int i = threadIdx.x; i < n; i += blockDim.x) {
+		const double x = v[i];
+		if (x > best) { best = x; bi = i; }                      // i grows within a thread: '>' keeps the smallest index of a tie
+		sum += x; sq = fma(x, x, sq);
+	}
+	for (int o = 16; o > 0; o >>= 1) {
+		const double ov = __shfl_xor_sync(0xffffffffu, best, o); const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+		if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
+		sum += __shfl_xor_sync(0xffffffffu, sum, o); sq += __shfl_xor_sync(0xffffffffu, sq, o);
+	}
+	if ((threadIdx.x & 31) == 0) { s_v[threadIdx.x >> 5] = best; s_i[threadIdx.x >> 5] = bi; s_s[threadIdx.x >> 5] = sum; s_q[threadIdx.x >> 5] = sq; }
+	__syncthreads();
+	if (threadIdx.x == 0) {
+		for (int w = 1; w < (int) (blockDim.x >> 5); w++) {
+			if (s_v[w] > best || (s_v[w] == best && s_i[w] < bi)) { best = s_v[w]; bi = s_i[w]; }
+			sum += s_s[w]; sq += s_q[w];
+		}
+		const double first = n > 0 ? v[0] : 0.0;
+		const int idx = (n <= 0 || first != first || bi == 0x7fffffff) ? 0 : bi;
+		double score = 0.0;
+		if (n > 0) {
+			const double mean = sum / n, var = sq / n - mean * mean, sd = var > 0.0 ? sqrt(var) : 0.0;
+			score = sd > 0.0 ? (v[idx] - mean) / sd : 0.0;
+		}
+		res[blockIdx.x].score = score; res[blockIdx.x].index = idx;
+	}
+}
 // first difference of magnitudes, out of place                          (superbandwidth.c:67-81)
 __global__ void k_abs_diff(const float2 *src, float2 *dst, unsigned long long pairs) {
 	for (unsigned long long i = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x; i < pairs; i += (unsigned long long) gridDim.x * blockDim.x) {
@@ -1077,6 +1125,30 @@ int tsdrgpu_crosscorrelation(tsdrgpu_ctx_t *ctx, void *stream_, float *d_a, floa
 	KL(ctx, "k_conj_mul", stream, k_conj_mul<<<grid1d(N, ctx->sm_count), 256, 0, stream>>>(reinterpret_cast<float2 *>(d_a), reinterpret_cast<const float2 *>(d_b), N));
 	return tsdrgpu_fft_internal(ctx, stream, reinterpret_cast<float2 *>(d_a), N, 1);
 }
+
+}  // extern "C"
+
+// one capture round of the scan (channelizer.cu): K captures of `size` magnitudes (capture c at d_caps + c * cap_stride) through the
+// batched autocorrelation (only the detector's two lag windows), the running means of every channel, then the peaks and scores
+int tsdrgpu_scan_round_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const float *d_caps, uint64_t cap_stride, uint32_t size,
+                                unsigned K, uint32_t rate, float *d_big, float2 *w0, float2 *w1, double *d_plots, uint64_t calls,
+                                TsdrScanPeak *d_res) {
+	int fmin, fmax, lmin, lmax;
+	tsdrgpu_frd_windows(rate, &fmin, &fmax, &lmin, &lmax);
+	const int flen = fmax - fmin, llen = lmax - lmin;
+	const uint32_t N = tsdrgpu_fft_getrealsize(size);
+	const bool skip_tail = (uint32_t) fmax <= N;
+	LagWindows win = LagWindows{0, 0, 0, 0};
+	if (skip_tail) win = LagWindows{(unsigned) fmin, (unsigned) fmax, (unsigned) lmin, (unsigned) lmax};
+	int rc = autocorrelation_batch(ctx, stream, d_big, 2ll * size, d_caps, (long long) cap_stride, size, K, skip_tail, win, WorkBufs{w0, w1});
+	if (rc) return rc;
+	KL(ctx, "k_accumulate_channels", stream, k_accumulate_channels<<<dim3(grid1d((unsigned long long) (flen + llen), ctx->sm_count), K), 256, 0, stream>>>(
+		d_plots, (long long) (flen + llen), (unsigned long long) calls, reinterpret_cast<const float2 *>(d_big), (long long) size, fmin, flen, lmin, llen));
+	KL(ctx, "k_plot_scores", stream, k_plot_scores<<<2 * K, 1024, 0, stream>>>(d_plots, (long long) (flen + llen), flen, llen, d_res));
+	return TSDRGPU_OK;
+}
+
+extern "C" {
 
 int tsdrgpu_accumulate(tsdrgpu_ctx_t *ctx, void *stream, double *d_out, uint64_t calls, const float *d_in, int startid, int length) {
 	BIND(ctx); ARG_TRY(ctx, d_out != NULL && d_in != NULL && length >= 0 && startid >= 0);

@@ -168,6 +168,9 @@ struct tsdrgpu_pipeline {
 	struct { double offset, bw; int D, ntaps; } tn_cfg; int tn_dirty;
 	tsdrgpu_tuner *tuner; int tn_on, tn_D; uint64_t tn_pos;           // what runs; tn_pos mirrors the tuner's input position
 	float *d_tout[4]; size_t tout_cap[4];                               // the tuner's output per staging slot (floats)
+	// scan (tsdrgpu_pipeline_set_scan): sc_cfg is the latest request (geo_mu), applied by the next process() call
+	struct { int K, Q; } sc_cfg; int sc_dirty;
+	tsdrgpu_scan_t *scan; int sc_on;
 	// delivery
 	pthread_t thread; pthread_mutex_t mu; pthread_cond_t cv_job, cv_done;
 	std::deque<FrameJob> jobs; int stop; uint64_t submitted, delivered;
@@ -593,6 +596,7 @@ int tsdrgpu_pipeline_create(tsdrgpu_ctx_t *ctx, const tsdrgpu_pipeline_config_t 
 	p->tn_cfg.offset = 0; p->tn_cfg.bw = 0; p->tn_cfg.D = 1; p->tn_cfg.ntaps = 0; p->tn_dirty = 0;
 	p->tuner = NULL; p->tn_on = 0; p->tn_D = 1; p->tn_pos = 0;
 	for (int i = 0; i < 4; i++) { p->d_tout[i] = NULL; p->tout_cap[i] = 0; }
+	p->sc_cfg.K = 0; p->sc_cfg.Q = 0; p->sc_dirty = 0; p->scan = NULL; p->sc_on = 0;
 	CU_TRY(ctx, cudaEventCreateWithFlags(&p->sb.ev, cudaEventDisableTiming));
 	memset(&p->stats, 0, sizeof p->stats);
 	CU_TRY(ctx, cudaStreamCreateWithFlags(&p->s_main, cudaStreamNonBlocking));
@@ -647,6 +651,7 @@ void tsdrgpu_pipeline_destroy(tsdrgpu_pipeline_t *p) {
 	for (int i = 0; i < 4; i++) if (p->d_raw[i]) cudaFree(p->d_raw[i]);
 	for (int i = 0; i < 4; i++) if (p->d_tout[i]) cudaFree(p->d_tout[i]);
 	tsdrgpu_tuner_destroy(p->tuner);
+	tsdrgpu_scan_destroy(p->scan);
 	if (p->d_argb_last) cudaFree(p->d_argb_last);
 	for (int s = 0; s < PL_SLOTS; s++) if (p->h_frames[s]) { cudaFreeHost(p->h_frames[s]); cudaFreeHost(p->h_results[s]); cudaFreeHost(p->h_report[s]); free(p->h_pll_rr[s]); }
 	cudaEventDestroy(p->ev_res);
@@ -681,6 +686,11 @@ int tsdrgpu_pipeline_set_samplerate(tsdrgpu_pipeline_t *p, uint32_t samplerate) 
 		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
 		p->tn_dirty = 1;
 	}
+	if (p->sc_cfg.K > 0) {                               // scanning: the filter bank is re-designed for the new rate (next process() call)
+		const int rc = tsdrgpu_channelizer_design(samplerate, p->sc_cfg.K, p->sc_cfg.Q, NULL, 0, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+		p->sc_dirty = 1;
+	}
 	p->samplerate = p->tn_cfg.bw > 0 ? samplerate / (uint32_t) p->tn_cfg.D : samplerate; p->samplerate_real = samplerate;
 	geometry_locked(p);
 	pthread_mutex_unlock(&p->geo_mu);
@@ -696,6 +706,27 @@ int tsdrgpu_pipeline_set_tuner(tsdrgpu_pipeline_t *p, double offset_hz, double b
 	p->tn_cfg.offset = offset_hz; p->tn_cfg.bw = bandwidth_hz > 0 ? bandwidth_hz : 0; p->tn_cfg.D = bandwidth_hz > 0 ? decimation : 1; p->tn_cfg.ntaps = ntaps;
 	p->tn_dirty = 1;
 	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_set_scan(tsdrgpu_pipeline_t *p, int channels, int taps_per_channel) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	pthread_mutex_lock(&p->geo_mu);
+	if (channels != 0) {
+		const int rc = tsdrgpu_channelizer_design(p->samplerate_real, channels, taps_per_channel, NULL, 0, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+	}
+	p->sc_cfg.K = channels; p->sc_cfg.Q = taps_per_channel;
+	p->sc_dirty = 1;
+	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_scan_results(tsdrgpu_pipeline_t *p, tsdrgpu_scan_channel_t *out, int cap, int *n) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	if (n) *n = 0;
+	if (!p->sc_on) return TSDRGPU_OK;
+	const int rc = tsdrgpu_scan_results(p->scan, p->s_ingest, out, cap);
+	if (rc) return rc;
+	if (n) *n = cap < p->sc_cfg.K ? cap : p->sc_cfg.K;
 	return TSDRGPU_OK;
 }
 // superbandwidth with one hop per GPU: devices[0] must be the pipeline's own device; n in {2, 4, 8} = number of hops.  n <= 1
@@ -758,6 +789,26 @@ static void superb_stop(tsdrgpu_pipeline *p) {                  // superbandwidt
 	geometry_locked(p);
 	pthread_mutex_unlock(&p->geo_mu);
 	if (p->tn_on) { p->tn_pos = 0; tsdrgpu_tuner_reset(p->tuner, p->s_ingest); }     // the tuner resumes from a clean start
+	if (p->sc_on) tsdrgpu_scan_reset(p->scan, p->s_ingest);                          // and so does the scan
+}
+
+// a scan (re)configuration, at the start of a process() call: the scan starts over; the pixel path does not notice
+static int scan_apply(tsdrgpu_pipeline *p) {
+	tsdrgpu_ctx_t *ctx = p->ctx;
+	int rc;
+	pthread_mutex_lock(&p->geo_mu);
+	const int dirty = p->sc_dirty, K = p->sc_cfg.K, Q = p->sc_cfg.Q;
+	const uint32_t fs = p->samplerate_real;
+	p->sc_dirty = 0;
+	pthread_mutex_unlock(&p->geo_mu);
+	if (!dirty) return TSDRGPU_OK;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_ingest));
+	if (K > 0) {
+		if (!p->scan && (rc = tsdrgpu_scan_create(ctx, &p->scan))) return rc;
+		if ((rc = tsdrgpu_scan_configure(p->scan, fs, K, Q))) return rc;      // resets
+		p->sc_on = 1;
+	} else p->sc_on = 0;
+	return TSDRGPU_OK;
 }
 
 // a tuner (re)configuration, at the start of a process() call: the stream starts over at the new internal rate
@@ -995,6 +1046,7 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	const uint64_t size2 = items_count >> 1;
 	int rc = tuner_apply(p);
 	if (rc) return rc;
+	if ((rc = scan_apply(p))) return rc;
 	pthread_mutex_lock(&p->geo_mu);
 	const int w = p->width, h = p->height; const double ptos = p->ptos;
 	pthread_mutex_unlock(&p->geo_mu);
@@ -1017,8 +1069,10 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	const bool drop_all = p->dev_drop.will_drop_all((uint32_t) n2);
 	const bool plots_on = !p->params[TSDRGPU_PARAM_AUTOCORR_PLOTS_OFF];
 	const bool need_data = n2 > 0 && (!drop_all || (plots_on && dropped != 0));
-	// the tuner sees every non-empty block, also one the drop compensation discards whole: its history and position stay continuous
-	const bool need_copy = tuned ? size2 > 0 : need_data;
+	// the tuner and the scan see every non-empty block, also one the drop compensation discards whole: their history and position
+	// stay continuous
+	const bool scanning = p->sc_on != 0;
+	const bool need_copy = (tuned || scanning) ? size2 > 0 : need_data;
 	const int ss = p->stage_slot;
 	float *stage = NULL, *d_in = NULL;
 	bool copy_issued = false;
@@ -1051,6 +1105,8 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 			}
 			p->stats.h2d_bytes += bytes;
 			d_in = stage;
+			// the scan reads the wideband block on this stream (covered by ev_used); its heavy part runs on a stream of its own
+			if (scanning && (rc = tsdrgpu_scan_run(p->scan, p->s_ingest, stage, size2, gap))) break;
 			if (tuned) {                                                       // shift, low-pass, decimate (tuner.cu)
 				if (p->tout_cap[ss] < 2 * n2 + 2) cudaStreamSynchronize(p->s_ingest);
 				if ((rc = grow(ctx, p->s_ingest, &p->d_tout[ss], &p->tout_cap[ss], 2 * n2 + 2, 0))) break;
@@ -1061,6 +1117,7 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 			if (need_data) { if ((rc = feed_capture(p, d_in, n2, dropped != 0))) break; }
 			else if (plots_on && dropped != 0) p->cap_fill = 0;
 		} else {
+			if (scanning && gap > 0 && (rc = tsdrgpu_scan_run(p->scan, p->s_ingest, NULL, 0, gap))) break;
 			if (tuned && gap > 0) {                                            // an empty block that only reports a loss
 				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, NULL, 0, gap, NULL, NULL, NULL))) break;
 				p->tn_pos += gap;

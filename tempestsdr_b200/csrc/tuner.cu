@@ -145,6 +145,26 @@ double bessel_i0(double x) {                                          // power s
 	return sum;
 }
 
+}  // namespace
+
+// scipy.signal.firwin(n, bandwidth / 2, window=('kaiser', beta), fs=fs): windowed sinc for 80 dB, designed in double, scaled to unit DC
+// gain, stored as float32.  The tuner and the channelizer both take their taps from here; each checks its own limits on n.
+void tsdrgpu_kaiser_lowpass_internal(uint32_t fs, double bandwidth_hz, int n, float *taps) {
+	const double cut = bandwidth_hz / (double) fs, alpha = 0.5 * (double) (n - 1), i0b = bessel_i0(TN_KAISER_BETA);
+	std::vector<double> h((size_t) n);
+	double sum = 0.0;
+	for (int i = 0; i < n; i++) {
+		const double m = (double) i - alpha, xm = cut * m;
+		const double sinc = xm == 0.0 ? 1.0 : sin(M_PI * xm) / (M_PI * xm);
+		const double rr = m / alpha, win = bessel_i0(TN_KAISER_BETA * sqrt(fmax(0.0, 1.0 - rr * rr))) / i0b;
+		h[i] = cut * sinc * win;
+		sum += h[i];
+	}
+	for (int i = 0; i < n; i++) taps[i] = (float) (h[i] / sum);
+}
+
+namespace {
+
 // validation + filter design shared by tsdrgpu_tuner_design and the tuner object (errors into ctx, or the thread's text)
 int tn_design(tsdrgpu_ctx_t *ctx, uint32_t fs, double offset_hz, double bandwidth_hz, int decimation, int ntaps, float *taps, int cap,
               int *ntaps_out, uint64_t *phase_inc) {
@@ -164,17 +184,7 @@ int tn_design(tsdrgpu_ctx_t *ctx, uint32_t fs, double offset_hz, double bandwidt
 	if (ntaps_out) *ntaps_out = n;
 	if (taps) {
 		if (cap < n) return tsdrgpu_fail(ctx, TSDRGPU_ECAPACITY, "tuner: the taps buffer is smaller than ntaps", cudaSuccess, __FILE__, __LINE__);
-		// scipy.signal.firwin(n, bandwidth / 2, window=('kaiser', beta), fs=fs): windowed sinc, scaled to unit DC gain
-		const double cut = bandwidth_hz / (double) fs, alpha = 0.5 * (double) (n - 1), i0b = bessel_i0(TN_KAISER_BETA);
-		double h[TN_MAX_TAPS], sum = 0.0;
-		for (int i = 0; i < n; i++) {
-			const double m = (double) i - alpha, xm = cut * m;
-			const double sinc = xm == 0.0 ? 1.0 : sin(M_PI * xm) / (M_PI * xm);
-			const double rr = m / alpha, win = bessel_i0(TN_KAISER_BETA * sqrt(fmax(0.0, 1.0 - rr * rr))) / i0b;
-			h[i] = cut * sinc * win;
-			sum += h[i];
-		}
-		for (int i = 0; i < n; i++) taps[i] = (float) (h[i] / sum);
+		tsdrgpu_kaiser_lowpass_internal(fs, bandwidth_hz, n, taps);
 	}
 	if (phase_inc) {                                                  // round(offset / fs * 2^64), two's complement
 		long double v = rintl((long double) offset_hz * 18446744073709551616.0L / (long double) fs);

@@ -70,6 +70,9 @@ struct tsdr_lib {
 	/* TSDR_TUNER=<offset_hz>,<bandwidth_hz>[,<decimation>[,<ntaps>]] (read by tsdr_readasync): the run demodulates that sub-band
 	 * only, at samplerate_real / tuner_d (1 = no tuner) */
 	double tn_offset, tn_bw; int tuner_d, tn_ntaps;
+	/* TSDR_SCAN=<channels>[,<taps_per_channel>] with TSDR_SCAN_FILE=<path> (read by tsdr_readasync): a frame-rate detector on every
+	 * sub-band of the capture; its table is written to the file as CSV when the run ends */
+	int sc_k, sc_q; const char *sc_file;
 };
 
 /* ---- error text: library-owned, NULL after a successful call (TSDRLibrary.c:136-159) ---------------------- */
@@ -186,6 +189,53 @@ static int parse_tuner(tsdr_lib_t *t, const char *text) {
 		return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
 	t->tn_offset = v[0]; t->tn_bw = v[1]; t->tuner_d = (int) v[2]; t->tn_ntaps = (int) v[3];
 	return TSDR_OK;
+}
+
+/* TSDR_SCAN: one or two integers separated by a comma, all of it consumed; checked against the plugin's rate by the channelizer's
+ * own rules, and only together with TSDR_SCAN_FILE */
+static int parse_scan(tsdr_lib_t *t, const char *text, const char *file) {
+	long v[2] = {0, 0};
+	int n = 0;
+	const char *c = text;
+	for (;;) {
+		char *e;
+		const long x = strtol(c, &e, 10);
+		if (e == c || n == 2) { n = -1; break; }
+		v[n++] = x; c = e;
+		while (*c == ' ') c++;
+		if (*c != ',') break;
+		c++;
+	}
+	if (n < 1 || *c != '\0' || v[0] < 1 || v[0] > 4096 || v[1] < 0 || v[1] > 4096)
+		return fail(t, "TSDR_SCAN: expected <channels>[,<taps_per_channel>] with integer values", TSDR_INVALID_PARAMETER_VALUE);
+	if (!file || !file[0]) return fail(t, "TSDR_SCAN: needs TSDR_SCAN_FILE=<path> for the table", TSDR_INVALID_PARAMETER_VALUE);
+	if (tsdrgpu_channelizer_design(t->samplerate_real, (int) v[0], (int) v[1], NULL, 0, NULL) != TSDRGPU_OK)
+		return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
+	t->sc_k = (int) v[0]; t->sc_q = (int) v[1]; t->sc_file = file;
+	return TSDR_OK;
+}
+
+/* the scan's table as CSV, one row per channel, highest frame_score first (ties: lower channel first) */
+struct scan_row { int channel; tsdrgpu_scan_channel_t r; };
+static int scan_cmp(const void *a, const void *b) {
+	const struct scan_row *x = (const struct scan_row *) a, *y = (const struct scan_row *) b;
+	if (x->r.frame_score != y->r.frame_score) return x->r.frame_score < y->r.frame_score ? 1 : -1;
+	return x->channel - y->channel;
+}
+static void write_scan(tsdr_lib_t *t, tsdrgpu_pipeline_t *p) {
+	tsdrgpu_scan_channel_t rec[256];
+	struct scan_row rows[256];
+	int n = 0;
+	if (tsdrgpu_pipeline_scan_results(p, rec, 256, &n) != TSDRGPU_OK) return;
+	for (int c = 0; c < n; c++) { rows[c].channel = c; rows[c].r = rec[c]; }
+	qsort(rows, (size_t) n, sizeof rows[0], scan_cmp);
+	FILE *f = fopen(t->sc_file, "w");
+	if (!f) return;
+	fprintf(f, "channel,offset_hz,rate,captures,fps,height,frame_score,line_score\n");
+	for (int i = 0; i < n; i++)
+		fprintf(f, "%d,%.3f,%u,%llu,%.6f,%d,%.6f,%.6f\n", rows[i].channel, rows[i].r.offset_hz, rows[i].r.rate, (unsigned long long) rows[i].r.captures,
+		        rows[i].r.fps, rows[i].r.height, rows[i].r.frame_score, rows[i].r.line_score);
+	fclose(f);
 }
 
 int tsdr_setbasefreq(tsdr_lib_t *t, uint32_t freq) {
@@ -358,7 +408,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	tsdr_reset(t);
 	t->nativerunning = 1; t->running = 1; t->gpu_failed = 0;
 	int status, pluginsfault = 0;
-	t->tuner_d = 1; t->tn_bw = 0.0;
+	t->tuner_d = 1; t->tn_bw = 0.0; t->sc_k = 0;
 	if ((status = tsdr_getsamplerate(t)) != TSDR_OK) goto end;
 	{
 		const char *tuner = getenv("TSDR_TUNER");
@@ -366,6 +416,8 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 			if ((status = parse_tuner(t, tuner)) != TSDR_OK) goto end;
 			set_internal_samplerate(t, t->samplerate_real / (uint32_t) t->tuner_d);     /* the geometry of the tuned sub-band */
 		}
+		const char *scan = getenv("TSDR_SCAN");
+		if (scan && scan[0] && (status = parse_scan(t, scan, getenv("TSDR_SCAN_FILE"))) != TSDR_OK) goto end;
 	}
 	if (t->width <= 0 || t->height <= 0 || (long long) t->width * t->height > MAX_PIXELS) {
 		status = fail(t, "The supplied height and the width are invalid!", TSDR_WRONG_VIDEOPARAMS);
@@ -417,6 +469,11 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 			tsdrgpu_pipeline_destroy(np);
 			goto end;
 		}
+		if (t->sc_k > 0 && tsdrgpu_pipeline_set_scan(np, t->sc_k, t->sc_q) != TSDRGPU_OK) {
+			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_INVALID_PARAMETER_VALUE);
+			tsdrgpu_pipeline_destroy(np);
+			goto end;
+		}
 		if (ndev > 1 && tsdrgpu_pipeline_set_superb_devices(np, devlist, ndev) != TSDRGPU_OK) {
 			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_CANNOT_OPEN_DEVICE);
 			tsdrgpu_pipeline_destroy(np);
@@ -447,6 +504,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 		}
 	}
 	tsdrgpu_pipeline_flush(t->pipe);
+	if (t->sc_k > 0) write_scan(t, t->pipe);
 	{
 		pthread_rwlock_wrlock(&t->pipe_lock);        /* no setter is inside the object any more, none can enter */
 		tsdrgpu_pipeline_t *p = t->pipe;

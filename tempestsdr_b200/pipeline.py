@@ -120,6 +120,19 @@ class Pipeline:
         at samplerate / decimation); bandwidth_hz <= 0 switches the tuner off.  Takes effect at the next process() call."""
         N.check(self._lib.tsdrgpu_pipeline_set_tuner(self._h, float(offset_hz), float(bandwidth_hz), int(decimation), int(ntaps)), self._ctx)
 
+    def set_scan(self, channels: int, taps_per_channel: int = 0) -> None:
+        """Run a frame-rate detector on each of `channels` sub-bands of the wideband blocks (0 switches it off).  Takes effect,
+        reset, at the next process() call; the pixel path is not affected."""
+        N.check(self._lib.tsdrgpu_pipeline_set_scan(self._h, int(channels), int(taps_per_channel)), self._ctx)
+
+    def scan_results(self):
+        """The scan's table: one dict per channel, sorted by frame_score, highest first (empty while no scan runs)."""
+        from .api import scan_table
+        recs = (N.ScanChannel * 256)()
+        n = C.c_int(0)
+        N.check(self._lib.tsdrgpu_pipeline_scan_results(self._h, recs, 256, C.byref(n)), self._ctx)
+        return scan_table(recs, n.value)
+
     def set_samplerate(self, samplerate: int) -> None:
         N.check(self._lib.tsdrgpu_pipeline_set_samplerate(self._h, int(samplerate)), self._ctx)
 
