@@ -416,6 +416,53 @@ TSDRGPU_API int  tsdrgpu_scan_results(tsdrgpu_scan_t *s, void *stream, tsdrgpu_s
  * synchronises */
 TSDRGPU_API int  tsdrgpu_scan_plots(tsdrgpu_scan_t *s, void *stream, double *h_plots, uint64_t cap, int *frame_len, int *line_len);
 
+/* ---------------------------------------------------------------------------- notch filter (stopbands ahead of the pixel path)
+ * Not in the reference: removes narrowband carriers from every block (DESIGN.md section 5.8).  Stopbands (f_j, w_j), j < n <= 32,
+ * in Hz in the capture's frame (that of tsdrgpu_pipeline_set_tuner's offset_hz and of the scan's table); L taps, L odd;
+ * delta(L) = (80 - 7.95) / (2.285 * 2 pi * (L - 1)) * fs, the transition width of the 80 dB Kaiser design.  The complex FIR is
+ *   h[m] = delta[m - (L-1)/2] - sum_j g_j[m] e^{2 pi i f_j (m - (L-1)/2) / fs},   g_j = the tuner's low-pass design at bandwidth w_j
+ * (scipy.signal.firwin(L, w_j / 2, window=('kaiser', 7.857), fs=fs)), designed in double, stored as float32.  Output
+ * y[n] = sum_k h[k] x~[n - k], x~ = the input with zeros before the stream and over every drop, n counted since the last reset:
+ * one output per input pair, the drop count passes through unchanged, the group delay is (L - 1) / 2 pairs.
+ * Configuration rules: 1 <= n <= 32, w_j > 0, |f_j| + w_j / 2 <= fs / 2, w_j >= 2 delta(L), neighbouring bands (sorted by
+ * frequency, also across +-fs/2) at least delta(L) apart edge to edge, L odd in 65..8193 (0 = the smallest odd L >= 65 that meets
+ * the width rule for the narrowest notch); anything else is TSDRGPU_EINVAL with a text naming the rule.
+ * Kernel: overlap-save with an FFT of N = the smallest power of two >= 2 (L - 1) in 1024..16384 points, hop N - (L - 1), segments at
+ * every multiple of the hop.  Cutting the stream at multiples of the hop gives bit-identical outputs; other cuts differ by FFT
+ * round-off in the segments a block boundary falls into. */
+typedef struct tsdrgpu_notch tsdrgpu_notch_t;
+/* host-only: validates; taps (NULL: validation only) receives the L complex float32 taps as interleaved re, im (cap >= L complex
+ * taps); *ntaps_out = L, *nfft_out = N (either may be NULL) */
+TSDRGPU_API int tsdrgpu_notch_design(uint32_t fs, int n, const double *centers, const double *widths, int ntaps, float *taps, int cap,
+                                     int *ntaps_out, int *nfft_out);
+TSDRGPU_API int  tsdrgpu_notch_create(tsdrgpu_ctx_t *ctx, tsdrgpu_notch_t **t);
+TSDRGPU_API void tsdrgpu_notch_destroy(tsdrgpu_notch_t *t);
+/* (re)design the filter and reset; synchronises the device */
+TSDRGPU_API int  tsdrgpu_notch_configure(tsdrgpu_notch_t *t, uint32_t fs, int n, const double *centers, const double *widths, int ntaps);
+TSDRGPU_API int  tsdrgpu_notch_reset(tsdrgpu_notch_t *t, void *stream);      /* position 0, history zero */
+/* d_iq: `pairs` interleaved I,Q pairs; d_out (not d_iq) receives *out_pairs = pairs pairs; *out_dropped = dropped_before.
+ * Asynchronous; the history of the last (L - 1) + (position mod hop) pairs is carried on the device. */
+TSDRGPU_API int  tsdrgpu_notch_run(tsdrgpu_notch_t *t, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before, float *d_out,
+                                   uint64_t *out_pairs, uint64_t *out_dropped);
+
+/* ---------------------------------------------------------------------------- power spectrum (Welch) of the capture
+ * Periodic Hann window of nfft points (a power of two in 64..16384), hop nfft / 2: segment s covers the absolute positions
+ * [s nfft/2, s nfft/2 + nfft) since the reset.  A segment that touches a dropped position is skipped; every complete segment's
+ * |X|^2 is added to per-bin double sums in segment order, so the result does not depend on how the stream is cut into blocks.
+ * Density = sum / (segments * fs * sum(w^2)), reported fft-shifted from -fs/2 to fs/2 - fs/nfft: with no drops,
+ * scipy.signal.welch(x, fs, window='hann', nperseg=nfft, noverlap=nfft/2, detrend=False, return_onesided=False,
+ * scaling='density'). */
+typedef struct tsdrgpu_spectrum tsdrgpu_spectrum_t;
+/* host-only: TSDRGPU_OK, or TSDRGPU_EINVAL with a text naming the rule */
+TSDRGPU_API int  tsdrgpu_spectrum_check(uint32_t fs, int nfft);
+TSDRGPU_API int  tsdrgpu_spectrum_create(tsdrgpu_ctx_t *ctx, tsdrgpu_spectrum_t **s);
+TSDRGPU_API void tsdrgpu_spectrum_destroy(tsdrgpu_spectrum_t *s);
+TSDRGPU_API int  tsdrgpu_spectrum_configure(tsdrgpu_spectrum_t *s, uint32_t fs, int nfft);      /* resets; synchronises */
+TSDRGPU_API int  tsdrgpu_spectrum_reset(tsdrgpu_spectrum_t *s, void *stream);
+TSDRGPU_API int  tsdrgpu_spectrum_run(tsdrgpu_spectrum_t *s, void *stream, const float *d_iq, uint64_t pairs, uint64_t dropped_before);
+/* min(cap, nfft) density values (fft-shifted) and the number of segments averaged; synchronises `stream` */
+TSDRGPU_API int  tsdrgpu_spectrum_results(tsdrgpu_spectrum_t *s, void *stream, double *h_psd, int cap, uint64_t *segments);
+
 /* ---------------------------------------------------------------------------- a1, a3, a5, a16, a17  streaming pipeline
  * replaces the body of process() (TSDRLibrary.c:264-298), decimatingthread / postprocessingthread /
  * videodecodingthread (TSDRLibrary.c:300-418) with their three rings (circbuff.c), dsp_dropped_compensation_*
@@ -490,6 +537,18 @@ TSDRGPU_API int  tsdrgpu_pipeline_set_tuner(tsdrgpu_pipeline_t *p, double offset
 TSDRGPU_API int  tsdrgpu_pipeline_set_scan(tsdrgpu_pipeline_t *p, int channels, int taps_per_channel);
 /* the scan's table (tsdrgpu_scan_results): *n = records written (0 while no scan runs); synchronises */
 TSDRGPU_API int  tsdrgpu_pipeline_scan_results(tsdrgpu_pipeline_t *p, tsdrgpu_scan_channel_t *out, int cap, int *n);
+/* The notch filter (see tsdrgpu_notch_*) on every non-empty block right after it reaches the device (any ingest format), after the
+ * spectrum and ahead of the scan and the tuner.  n = 0 switches it off (the default).  Checked against the current rate at once
+ * (TSDRGPU_EINVAL + text); takes effect at the next process() call, which then starts over behind it: notch, tuner and scan at
+ * position 0, samples and pixels waiting discarded, resampler, frame stage and frame-rate detector reset.  Superbandwidth mode
+ * bypasses it and resumes it, reset, when it ends.  set_samplerate re-designs the filter or rejects the rate. */
+TSDRGPU_API int  tsdrgpu_pipeline_set_notches(tsdrgpu_pipeline_t *p, int n, const double *centers, const double *widths, int ntaps);
+/* The power spectrum (see tsdrgpu_spectrum_*) of every non-empty block as received, at the capture's rate.  nfft = 0 switches it
+ * off (the default).  Takes effect, reset, at the next process() call; the pixel path is not affected.  Superbandwidth mode
+ * pauses it; it resumes, reset, when that mode ends. */
+TSDRGPU_API int  tsdrgpu_pipeline_set_spectrum(tsdrgpu_pipeline_t *p, int nfft);
+/* the spectrum (tsdrgpu_spectrum_results): *n = values written (0 while no spectrum runs), *segments averaged; synchronises */
+TSDRGPU_API int  tsdrgpu_pipeline_spectrum(tsdrgpu_pipeline_t *p, double *out, int cap, int *n, uint64_t *segments);
 /* superbandwidth mode (PARAM_AUTOCORR_SUPERRESOLUTION = 1; superb_run, superbandwidth.c:179-254) retunes the front end
  * between hops through this callback; without it the hops are recorded at one frequency */
 TSDRGPU_API int  tsdrgpu_pipeline_set_retune(tsdrgpu_pipeline_t *p, tsdrgpu_retune_cb cb);

@@ -181,6 +181,24 @@ _SIGS = {
     "tsdrgpu_scan_plots": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "tsdrgpu_pipeline_set_scan": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
     "tsdrgpu_pipeline_scan_results": (C.c_int, [C.c_void_p, C.POINTER(ScanChannel), C.c_int, C.POINTER(C.c_int)]),
+    "tsdrgpu_notch_design": (C.c_int, [C.c_uint32, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(C.c_int),
+                                       C.POINTER(C.c_int)]),
+    "tsdrgpu_notch_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "tsdrgpu_notch_destroy": (None, [C.c_void_p]),
+    "tsdrgpu_notch_configure": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "tsdrgpu_notch_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tsdrgpu_notch_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_void_p,
+                                    C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]),
+    "tsdrgpu_spectrum_check": (C.c_int, [C.c_uint32, C.c_int]),
+    "tsdrgpu_spectrum_create": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
+    "tsdrgpu_spectrum_destroy": (None, [C.c_void_p]),
+    "tsdrgpu_spectrum_configure": (C.c_int, [C.c_void_p, C.c_uint32, C.c_int]),
+    "tsdrgpu_spectrum_reset": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "tsdrgpu_spectrum_run": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64]),
+    "tsdrgpu_spectrum_results": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_uint64)]),
+    "tsdrgpu_pipeline_set_notches": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int]),
+    "tsdrgpu_pipeline_set_spectrum": (C.c_int, [C.c_void_p, C.c_int]),
+    "tsdrgpu_pipeline_spectrum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_uint64)]),
     "tsdrgpu_pipeline_set_retune": (C.c_int, [C.c_void_p, RETUNE_CB]),
     "tsdrgpu_pipeline_set_motionblur": (C.c_int, [C.c_void_p, C.c_float]),
     "tsdrgpu_pipeline_set_host_registration": (C.c_int, [C.c_void_p, C.c_int]),

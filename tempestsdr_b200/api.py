@@ -192,6 +192,12 @@ class Context:
     def scan(self) -> "Scan":
         return Scan(self)
 
+    def notch(self) -> "Notch":
+        return Notch(self)
+
+    def spectrum(self) -> "Spectrum":
+        return Spectrum(self)
+
 
 def tuner_design(fs: int, offset_hz: float, bandwidth_hz: float, decimation: int = 1, ntaps: int = 0) -> Tuple[np.ndarray, int]:
     """tsdrgpu_tuner_design (host only): the float32 taps and the 64-bit phase increment round(offset / fs * 2^64) (as an
@@ -555,3 +561,116 @@ class FrameRateDetector:
                                                    fp.ctypes.data_as(C.c_void_p) if copy_out else None, fmax - fmin,
                                                    lp.ctypes.data_as(C.c_void_p) if copy_out else None, lmax - lmin, C.byref(calls)))
         return (fmin, fp), (lmin, lp), calls.value
+
+
+def _bands(centers: Sequence[float], widths: Sequence[float]):
+    c = np.ascontiguousarray(centers, dtype=np.float64)
+    w = np.ascontiguousarray(widths, dtype=np.float64)
+    assert c.shape == w.shape and c.ndim == 1, "one width per center"
+    return c, w
+
+
+def notch_design(fs: int, centers: Sequence[float], widths: Sequence[float], ntaps: int = 0) -> Tuple[np.ndarray, int]:
+    """tsdrgpu_notch_design (host only): the complex64 taps of the notch filter and its FFT size N.  Raises TsdrGpuError naming
+    the violated rule."""
+    c, w = _bands(centers, widths)
+    n, nfft = C.c_int(0), C.c_int(0)
+    N.check(N.lib().tsdrgpu_notch_design(int(fs), c.size, c.ctypes.data_as(C.c_void_p), w.ctypes.data_as(C.c_void_p), int(ntaps),
+                                         None, 0, C.byref(n), C.byref(nfft)))
+    taps = np.zeros(2 * n.value, np.float32)
+    N.check(N.lib().tsdrgpu_notch_design(int(fs), c.size, c.ctypes.data_as(C.c_void_p), w.ctypes.data_as(C.c_void_p), int(ntaps),
+                                         taps.ctypes.data_as(C.c_void_p), n.value, None, None))
+    return taps.view(np.complex64).copy(), nfft.value
+
+
+class Notch:
+    """The notch filter (tsdrgpu_notch_*): removes the stopbands (center, width) from the stream, one output per input pair."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        h = C.c_void_p()
+        ctx.chk(ctx._lib.tsdrgpu_notch_create(ctx._h, C.byref(h)))
+        self._h = h
+        self.config = None
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx._lib.tsdrgpu_notch_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def configure(self, fs: int, centers: Sequence[float], widths: Sequence[float], ntaps: int = 0) -> None:
+        """Design the filter for these stopbands and reset (position 0, history zero)."""
+        c, w = _bands(centers, widths)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_notch_configure(self._h, int(fs), c.size, c.ctypes.data_as(C.c_void_p), w.ctypes.data_as(C.c_void_p),
+                                                           int(ntaps)))
+        self.config = (int(fs), c.copy(), w.copy(), int(ntaps))
+
+    def taps(self) -> np.ndarray:
+        """The complex64 taps in use."""
+        assert self.config is not None, "configure() first"
+        return notch_design(*self.config)[0]
+
+    @property
+    def nfft(self) -> int:
+        assert self.config is not None, "configure() first"
+        return notch_design(*self.config)[1]
+
+    def reset(self) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_notch_reset(self._h, self.ctx.stream))
+
+    def run(self, x: torch.Tensor, dropped: int = 0) -> Tuple[torch.Tensor, int]:
+        """x: interleaved I,Q float32 on the device (the next block of the stream), preceded by `dropped` lost pairs.
+        Returns (the filtered I,Q pairs, as many as x holds, and the drop count, unchanged)."""
+        pairs = x.numel() // 2
+        out = torch.empty(2 * pairs, dtype=torch.float32, device=self.ctx.device)
+        o, od = C.c_uint64(0), C.c_uint64(0)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_notch_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped),
+                                                     out.data_ptr() if pairs else None, C.byref(o), C.byref(od)))
+        return out[: 2 * o.value], od.value
+
+
+def spectrum_freqs(fs: int, nfft: int) -> np.ndarray:
+    """The frequencies of the spectrum's bins, fft-shifted: -fs/2 .. fs/2 - fs/nfft."""
+    return (np.arange(nfft) - nfft // 2) * (fs / max(nfft, 1))
+
+
+class Spectrum:
+    """Welch's power spectral density of the stream (tsdrgpu_spectrum_*): Hann window, half-overlapping segments, drops skipped."""
+
+    def __init__(self, ctx: Context):
+        self.ctx = ctx
+        h = C.c_void_p()
+        ctx.chk(ctx._lib.tsdrgpu_spectrum_create(ctx._h, C.byref(h)))
+        self._h = h
+        self.config = None
+
+    def __del__(self):
+        try:
+            if self._h:
+                self.ctx._lib.tsdrgpu_spectrum_destroy(self._h)
+                self._h = None
+        except Exception:
+            pass
+
+    def configure(self, fs: int, nfft: int = 4096) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_spectrum_configure(self._h, int(fs), int(nfft)))
+        self.config = (int(fs), int(nfft))
+
+    def reset(self) -> None:
+        self.ctx.chk(self.ctx._lib.tsdrgpu_spectrum_reset(self._h, self.ctx.stream))
+
+    def run(self, x: torch.Tensor, dropped: int = 0) -> None:
+        pairs = x.numel() // 2
+        self.ctx.chk(self.ctx._lib.tsdrgpu_spectrum_run(self._h, self.ctx.stream, _f32(x).data_ptr() if pairs else None, pairs, int(dropped)))
+
+    def result(self) -> Tuple[np.ndarray, np.ndarray, int]:
+        """(frequencies in Hz, density per Hz, segments averaged), fft-shifted."""
+        assert self.config is not None, "configure() first"
+        fs, nfft = self.config
+        psd = np.zeros(nfft, np.float64)
+        segs = C.c_uint64(0)
+        self.ctx.chk(self.ctx._lib.tsdrgpu_spectrum_results(self._h, self.ctx.stream, psd.ctypes.data_as(C.c_void_p), nfft, C.byref(segs)))
+        return spectrum_freqs(fs, nfft), psd, segs.value

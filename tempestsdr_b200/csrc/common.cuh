@@ -94,6 +94,8 @@ int tsdrgpu_ifft_abs_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, float2 *d
 int tsdrgpu_argmax_mag_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const float2 *x, unsigned n, void *d_part, int *d_result);
 // the tuner's filter designer (tuner.cu), shared with the channelizer: n float32 taps of a Kaiser-windowed sinc low-pass
 void tsdrgpu_kaiser_lowpass_internal(uint32_t fs, double bandwidth_hz, int n, float *taps);
+// the same design before the rounding to float32 (the notch filter's low-pass prototypes)
+void tsdrgpu_kaiser_lowpass_double_internal(uint32_t fs, double bandwidth_hz, int n, double *taps);
 // the scan's per-plot result (fft.cu's k_plot_scores): first strict maximum and (max - mean) / std
 struct TsdrScanPeak { double score; int32_t index, pad; };
 int tsdrgpu_scan_round_internal(tsdrgpu_ctx_t *ctx, cudaStream_t stream, const float *d_caps, uint64_t cap_stride, uint32_t size,

@@ -171,6 +171,13 @@ struct tsdrgpu_pipeline {
 	// scan (tsdrgpu_pipeline_set_scan): sc_cfg is the latest request (geo_mu), applied by the next process() call
 	struct { int K, Q; } sc_cfg; int sc_dirty;
 	tsdrgpu_scan_t *scan; int sc_on;
+	// notch filter (tsdrgpu_pipeline_set_notches): nt_cfg is the latest request (geo_mu), applied by the next process() call
+	struct { int n, ntaps; double centers[32], widths[32]; } nt_cfg; int nt_dirty;
+	tsdrgpu_notch_t *notch; int nt_on;
+	float *d_nout[4]; size_t nout_cap[4];                               // the notch's output per staging slot (floats)
+	// spectrum (tsdrgpu_pipeline_set_spectrum): sp_nfft is the latest request (geo_mu), applied by the next process() call
+	int sp_nfft, sp_dirty;
+	tsdrgpu_spectrum_t *spectrum; int sp_on;
 	// delivery
 	pthread_t thread; pthread_mutex_t mu; pthread_cond_t cv_job, cv_done;
 	std::deque<FrameJob> jobs; int stop; uint64_t submitted, delivered;
@@ -597,6 +604,9 @@ int tsdrgpu_pipeline_create(tsdrgpu_ctx_t *ctx, const tsdrgpu_pipeline_config_t 
 	p->tuner = NULL; p->tn_on = 0; p->tn_D = 1; p->tn_pos = 0;
 	for (int i = 0; i < 4; i++) { p->d_tout[i] = NULL; p->tout_cap[i] = 0; }
 	p->sc_cfg.K = 0; p->sc_cfg.Q = 0; p->sc_dirty = 0; p->scan = NULL; p->sc_on = 0;
+	memset(&p->nt_cfg, 0, sizeof p->nt_cfg); p->nt_dirty = 0; p->notch = NULL; p->nt_on = 0;
+	for (int i = 0; i < 4; i++) { p->d_nout[i] = NULL; p->nout_cap[i] = 0; }
+	p->sp_nfft = 0; p->sp_dirty = 0; p->spectrum = NULL; p->sp_on = 0;
 	CU_TRY(ctx, cudaEventCreateWithFlags(&p->sb.ev, cudaEventDisableTiming));
 	memset(&p->stats, 0, sizeof p->stats);
 	CU_TRY(ctx, cudaStreamCreateWithFlags(&p->s_main, cudaStreamNonBlocking));
@@ -652,6 +662,9 @@ void tsdrgpu_pipeline_destroy(tsdrgpu_pipeline_t *p) {
 	for (int i = 0; i < 4; i++) if (p->d_tout[i]) cudaFree(p->d_tout[i]);
 	tsdrgpu_tuner_destroy(p->tuner);
 	tsdrgpu_scan_destroy(p->scan);
+	for (int i = 0; i < 4; i++) if (p->d_nout[i]) cudaFree(p->d_nout[i]);
+	tsdrgpu_notch_destroy(p->notch);
+	tsdrgpu_spectrum_destroy(p->spectrum);
 	if (p->d_argb_last) cudaFree(p->d_argb_last);
 	for (int s = 0; s < PL_SLOTS; s++) if (p->h_frames[s]) { cudaFreeHost(p->h_frames[s]); cudaFreeHost(p->h_results[s]); cudaFreeHost(p->h_report[s]); free(p->h_pll_rr[s]); }
 	cudaEventDestroy(p->ev_res);
@@ -691,6 +704,12 @@ int tsdrgpu_pipeline_set_samplerate(tsdrgpu_pipeline_t *p, uint32_t samplerate) 
 		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
 		p->sc_dirty = 1;
 	}
+	if (p->nt_cfg.n > 0) {                               // notched: the filter is re-designed for the new rate (next process() call)
+		const int rc = tsdrgpu_notch_design(samplerate, p->nt_cfg.n, p->nt_cfg.centers, p->nt_cfg.widths, p->nt_cfg.ntaps, NULL, 0, NULL, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+		p->nt_dirty = 1;
+	}
+	if (p->sp_nfft > 0) p->sp_dirty = 1;                 // the spectrum starts over at the new rate
 	p->samplerate = p->tn_cfg.bw > 0 ? samplerate / (uint32_t) p->tn_cfg.D : samplerate; p->samplerate_real = samplerate;
 	geometry_locked(p);
 	pthread_mutex_unlock(&p->geo_mu);
@@ -727,6 +746,40 @@ int tsdrgpu_pipeline_scan_results(tsdrgpu_pipeline_t *p, tsdrgpu_scan_channel_t 
 	const int rc = tsdrgpu_scan_results(p->scan, p->s_ingest, out, cap);
 	if (rc) return rc;
 	if (n) *n = cap < p->sc_cfg.K ? cap : p->sc_cfg.K;
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_set_notches(tsdrgpu_pipeline_t *p, int n, const double *centers, const double *widths, int ntaps) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	pthread_mutex_lock(&p->geo_mu);
+	if (n != 0) {
+		const int rc = tsdrgpu_notch_design(p->samplerate_real, n, centers, widths, ntaps, NULL, 0, NULL, NULL);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+		for (int j = 0; j < n; j++) { p->nt_cfg.centers[j] = centers[j]; p->nt_cfg.widths[j] = widths[j]; }
+	}
+	p->nt_cfg.n = n; p->nt_cfg.ntaps = ntaps;
+	p->nt_dirty = 1;
+	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_set_spectrum(tsdrgpu_pipeline_t *p, int nfft) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	pthread_mutex_lock(&p->geo_mu);
+	if (nfft != 0) {
+		const int rc = tsdrgpu_spectrum_check(p->samplerate_real, nfft);
+		if (rc) { pthread_mutex_unlock(&p->geo_mu); snprintf(p->ctx->err, sizeof p->ctx->err, "%s", tsdrgpu_last_error(NULL)); return rc; }
+	}
+	p->sp_nfft = nfft; p->sp_dirty = 1;
+	pthread_mutex_unlock(&p->geo_mu);
+	return TSDRGPU_OK;
+}
+int tsdrgpu_pipeline_spectrum(tsdrgpu_pipeline_t *p, double *out, int cap, int *n, uint64_t *segments) {
+	ARG_TRY((tsdrgpu_ctx_t *) NULL, p != NULL);
+	if (n) *n = 0;
+	if (segments) *segments = 0;
+	if (!p->sp_on) return TSDRGPU_OK;
+	const int rc = tsdrgpu_spectrum_results(p->spectrum, p->s_ingest, out, cap, segments);
+	if (rc) return rc;
+	if (n) *n = cap < p->sp_nfft ? cap : p->sp_nfft;
 	return TSDRGPU_OK;
 }
 // superbandwidth with one hop per GPU: devices[0] must be the pipeline's own device; n in {2, 4, 8} = number of hops.  n <= 1
@@ -790,6 +843,59 @@ static void superb_stop(tsdrgpu_pipeline *p) {                  // superbandwidt
 	pthread_mutex_unlock(&p->geo_mu);
 	if (p->tn_on) { p->tn_pos = 0; tsdrgpu_tuner_reset(p->tuner, p->s_ingest); }     // the tuner resumes from a clean start
 	if (p->sc_on) tsdrgpu_scan_reset(p->scan, p->s_ingest);                          // and so does the scan
+	if (p->nt_on) tsdrgpu_notch_reset(p->notch, p->s_ingest);                        // and the notch
+	if (p->sp_on) tsdrgpu_spectrum_reset(p->spectrum, p->s_ingest);                  // and the spectrum
+}
+
+// a spectrum (re)configuration, at the start of a process() call: the spectrum starts over; the pixel path does not notice
+static int spectrum_apply(tsdrgpu_pipeline *p) {
+	tsdrgpu_ctx_t *ctx = p->ctx;
+	int rc;
+	pthread_mutex_lock(&p->geo_mu);
+	const int dirty = p->sp_dirty, nfft = p->sp_nfft;
+	const uint32_t fs = p->samplerate_real;
+	p->sp_dirty = 0;
+	pthread_mutex_unlock(&p->geo_mu);
+	if (!dirty) return TSDRGPU_OK;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_ingest));
+	if (nfft > 0) {
+		if (!p->spectrum && (rc = tsdrgpu_spectrum_create(ctx, &p->spectrum))) return rc;
+		if ((rc = tsdrgpu_spectrum_configure(p->spectrum, fs, nfft))) return rc;      // resets
+		p->sp_on = 1;
+	} else p->sp_on = 0;
+	return TSDRGPU_OK;
+}
+
+// a notch (re)configuration, at the start of a process() call: the stream starts over behind the notch as a new pipeline would
+static int notch_apply(tsdrgpu_pipeline *p) {
+	tsdrgpu_ctx_t *ctx = p->ctx;
+	int rc;
+	pthread_mutex_lock(&p->geo_mu);
+	const int dirty = p->nt_dirty, n = p->nt_cfg.n, ntaps = p->nt_cfg.ntaps;
+	double centers[32], widths[32];
+	for (int j = 0; j < n; j++) { centers[j] = p->nt_cfg.centers[j]; widths[j] = p->nt_cfg.widths[j]; }
+	const uint32_t fs = p->samplerate_real;
+	p->nt_dirty = 0;
+	pthread_mutex_unlock(&p->geo_mu);
+	if (!dirty) return TSDRGPU_OK;
+	if ((rc = tsdrgpu_framestage_join(p->fs, p->s_main))) return rc;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_copy)); CU_TRY(ctx, cudaStreamSynchronize(p->s_ingest));
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_main)); CU_TRY(ctx, cudaStreamSynchronize(p->s_out));
+	if (n > 0) {
+		if (!p->notch && (rc = tsdrgpu_notch_create(ctx, &p->notch))) return rc;
+		if ((rc = tsdrgpu_notch_configure(p->notch, fs, n, centers, widths, ntaps))) return rc;      // resets
+		p->nt_on = 1;
+	} else p->nt_on = 0;
+	if (p->tn_on) { p->tn_pos = 0; if ((rc = tsdrgpu_tuner_reset(p->tuner, p->s_ingest))) return rc; }
+	if (p->sc_on && (rc = tsdrgpu_scan_reset(p->scan, p->s_ingest))) return rc;
+	p->decim_fill = 0; p->decim_read = 0; p->decim_elem = 2; p->pix_fill = 0; p->pix_read = 0; p->cap_fill = 0;
+	p->dev_drop = DropComp(); p->pix_drop = DropComp();
+	if ((rc = tsdrgpu_resampler_reset(p->rs, p->s_main))) return rc;
+	if ((rc = tsdrgpu_framestage_reset(p->fs, p->s_main))) return rc;
+	if ((rc = tsdrgpu_frd_reset(p->frd))) return rc;
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_main));
+	CU_TRY(ctx, cudaStreamSynchronize(p->s_ingest));
+	return TSDRGPU_OK;
 }
 
 // a scan (re)configuration, at the start of a process() call: the scan starts over; the pixel path does not notice
@@ -1047,6 +1153,8 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	int rc = tuner_apply(p);
 	if (rc) return rc;
 	if ((rc = scan_apply(p))) return rc;
+	if ((rc = notch_apply(p))) return rc;
+	if ((rc = spectrum_apply(p))) return rc;
 	pthread_mutex_lock(&p->geo_mu);
 	const int w = p->width, h = p->height; const double ptos = p->ptos;
 	pthread_mutex_unlock(&p->geo_mu);
@@ -1071,8 +1179,8 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 	const bool need_data = n2 > 0 && (!drop_all || (plots_on && dropped != 0));
 	// the tuner and the scan see every non-empty block, also one the drop compensation discards whole: their history and position
 	// stay continuous
-	const bool scanning = p->sc_on != 0;
-	const bool need_copy = (tuned || scanning) ? size2 > 0 : need_data;
+	const bool scanning = p->sc_on != 0, notched = p->nt_on != 0, spectrum = p->sp_on != 0;
+	const bool need_copy = (tuned || scanning || notched || spectrum) ? size2 > 0 : need_data;
 	const int ss = p->stage_slot;
 	float *stage = NULL, *d_in = NULL;
 	bool copy_issued = false;
@@ -1104,19 +1212,30 @@ static int process_impl(tsdrgpu_pipeline_t *p, const void *h_iq, int fmt, uint64
 				if ((e = cudaGetLastError()) != cudaSuccess) { rc = tsdrgpu_fail(ctx, TSDRGPU_ECUDA, "kernel launch", e, __FILE__, __LINE__); break; }
 			}
 			p->stats.h2d_bytes += bytes;
-			d_in = stage;
+			// the spectrum reads the block as received, on this stream (covered by ev_used)
+			if (spectrum && (rc = tsdrgpu_spectrum_run(p->spectrum, p->s_ingest, stage, size2, gap))) break;
+			float *wide = stage;                                               // what the scan and the tuner read
+			if (notched) {                                                     // the stopbands removed (notch.cu)
+				if (p->nout_cap[ss] < 2 * size2) cudaStreamSynchronize(p->s_ingest);
+				if ((rc = grow(ctx, p->s_ingest, &p->d_nout[ss], &p->nout_cap[ss], 2 * size2, 0))) break;
+				if ((rc = tsdrgpu_notch_run(p->notch, p->s_ingest, stage, size2, gap, p->d_nout[ss], NULL, NULL))) break;
+				wide = p->d_nout[ss];
+			}
+			d_in = wide;
 			// the scan reads the wideband block on this stream (covered by ev_used); its heavy part runs on a stream of its own
-			if (scanning && (rc = tsdrgpu_scan_run(p->scan, p->s_ingest, stage, size2, gap))) break;
+			if (scanning && (rc = tsdrgpu_scan_run(p->scan, p->s_ingest, wide, size2, gap))) break;
 			if (tuned) {                                                       // shift, low-pass, decimate (tuner.cu)
 				if (p->tout_cap[ss] < 2 * n2 + 2) cudaStreamSynchronize(p->s_ingest);
 				if ((rc = grow(ctx, p->s_ingest, &p->d_tout[ss], &p->tout_cap[ss], 2 * n2 + 2, 0))) break;
-				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, stage, size2, gap, p->d_tout[ss], NULL, NULL))) break;
+				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, wide, size2, gap, p->d_tout[ss], NULL, NULL))) break;
 				p->tn_pos += gap + size2;
 				d_in = p->d_tout[ss];
 			}
 			if (need_data) { if ((rc = feed_capture(p, d_in, n2, dropped != 0))) break; }
 			else if (plots_on && dropped != 0) p->cap_fill = 0;
 		} else {
+			if (spectrum && gap > 0 && (rc = tsdrgpu_spectrum_run(p->spectrum, p->s_ingest, NULL, 0, gap))) break;
+			if (notched && gap > 0 && (rc = tsdrgpu_notch_run(p->notch, p->s_ingest, NULL, 0, gap, NULL, NULL, NULL))) break;
 			if (scanning && gap > 0 && (rc = tsdrgpu_scan_run(p->scan, p->s_ingest, NULL, 0, gap))) break;
 			if (tuned && gap > 0) {                                            // an empty block that only reports a loss
 				if ((rc = tsdrgpu_tuner_run(p->tuner, p->s_ingest, NULL, 0, gap, NULL, NULL, NULL))) break;

@@ -147,20 +147,26 @@ double bessel_i0(double x) {                                          // power s
 
 }  // namespace
 
-// scipy.signal.firwin(n, bandwidth / 2, window=('kaiser', beta), fs=fs): windowed sinc for 80 dB, designed in double, scaled to unit DC
-// gain, stored as float32.  The tuner and the channelizer both take their taps from here; each checks its own limits on n.
-void tsdrgpu_kaiser_lowpass_internal(uint32_t fs, double bandwidth_hz, int n, float *taps) {
+// scipy.signal.firwin(n, bandwidth / 2, window=('kaiser', beta), fs=fs): windowed sinc for 80 dB, designed in double and scaled to
+// unit DC gain.  The tuner and the channelizer store it as float32 (tsdrgpu_kaiser_lowpass_internal), the notch builds on the
+// doubles; each checks its own limits on n.
+void tsdrgpu_kaiser_lowpass_double_internal(uint32_t fs, double bandwidth_hz, int n, double *taps) {
 	const double cut = bandwidth_hz / (double) fs, alpha = 0.5 * (double) (n - 1), i0b = bessel_i0(TN_KAISER_BETA);
-	std::vector<double> h((size_t) n);
 	double sum = 0.0;
 	for (int i = 0; i < n; i++) {
 		const double m = (double) i - alpha, xm = cut * m;
 		const double sinc = xm == 0.0 ? 1.0 : sin(M_PI * xm) / (M_PI * xm);
 		const double rr = m / alpha, win = bessel_i0(TN_KAISER_BETA * sqrt(fmax(0.0, 1.0 - rr * rr))) / i0b;
-		h[i] = cut * sinc * win;
-		sum += h[i];
+		taps[i] = cut * sinc * win;
+		sum += taps[i];
 	}
-	for (int i = 0; i < n; i++) taps[i] = (float) (h[i] / sum);
+	for (int i = 0; i < n; i++) taps[i] /= sum;
+}
+
+void tsdrgpu_kaiser_lowpass_internal(uint32_t fs, double bandwidth_hz, int n, float *taps) {
+	std::vector<double> h((size_t) n);
+	tsdrgpu_kaiser_lowpass_double_internal(fs, bandwidth_hz, n, h.data());
+	for (int i = 0; i < n; i++) taps[i] = (float) h[i];
 }
 
 namespace {

@@ -17,6 +17,7 @@
 #include "../../include/tsdrgpu.h"
 
 #include <dlfcn.h>
+#include <math.h>
 #include <pthread.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -73,6 +74,12 @@ struct tsdr_lib {
 	/* TSDR_SCAN=<channels>[,<taps_per_channel>] with TSDR_SCAN_FILE=<path> (read by tsdr_readasync): a frame-rate detector on every
 	 * sub-band of the capture; its table is written to the file as CSV when the run ends */
 	int sc_k, sc_q; const char *sc_file;
+	/* TSDR_NOTCH=<center_hz>:<width_hz>[,<center_hz>:<width_hz>...] with an optional TSDR_NOTCH_TAPS=<ntaps> (read by
+	 * tsdr_readasync): those stopbands are removed from every block before anything else reads it */
+	int nt_n, nt_taps; double nt_centers[32], nt_widths[32];
+	/* TSDR_SPECTRUM=<nfft> with TSDR_SPECTRUM_FILE=<path> (read by tsdr_readasync): the capture's power spectrum, written to the file
+	 * as CSV when the run ends */
+	int sp_nfft; const char *sp_file;
 };
 
 /* ---- error text: library-owned, NULL after a successful call (TSDRLibrary.c:136-159) ---------------------- */
@@ -213,6 +220,61 @@ static int parse_scan(tsdr_lib_t *t, const char *text, const char *file) {
 		return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
 	t->sc_k = (int) v[0]; t->sc_q = (int) v[1]; t->sc_file = file;
 	return TSDR_OK;
+}
+
+/* TSDR_NOTCH: center:width pairs separated by commas, all of it consumed; TSDR_NOTCH_TAPS: one integer.  Checked against the
+ * plugin's rate by the notch's own rules */
+static int parse_notch(tsdr_lib_t *t, const char *text, const char *taps) {
+	int n = 0;
+	const char *c = text;
+	for (;;) {
+		char *e;
+		if (n == 32) return fail(t, "TSDR_NOTCH: at most 32 notches", TSDR_INVALID_PARAMETER_VALUE);
+		const double f = strtod(c, &e);
+		if (e == c || *e != ':') { n = -1; break; }
+		c = e + 1;
+		const double w = strtod(c, &e);
+		if (e == c) { n = -1; break; }
+		t->nt_centers[n] = f; t->nt_widths[n] = w; n++; c = e;
+		while (*c == ' ') c++;
+		if (*c != ',') break;
+		c++;
+	}
+	if (n < 1 || *c != '\0') return fail(t, "TSDR_NOTCH: expected <center_hz>:<width_hz>[,<center_hz>:<width_hz>...]", TSDR_INVALID_PARAMETER_VALUE);
+	long L = 0;
+	if (taps && taps[0]) {
+		char *e;
+		L = strtol(taps, &e, 10);
+		if (e == taps || *e != '\0' || L < 1 || L > 1000000) return fail(t, "TSDR_NOTCH_TAPS: expected an odd integer ntaps", TSDR_INVALID_PARAMETER_VALUE);
+	}
+	if (tsdrgpu_notch_design(t->samplerate_real, n, t->nt_centers, t->nt_widths, (int) L, NULL, 0, NULL, NULL) != TSDRGPU_OK)
+		return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
+	t->nt_n = n; t->nt_taps = (int) L;
+	return TSDR_OK;
+}
+
+/* TSDR_SPECTRUM: one integer, only together with TSDR_SPECTRUM_FILE */
+static int parse_spectrum(tsdr_lib_t *t, const char *text, const char *file) {
+	char *e;
+	const long v = strtol(text, &e, 10);
+	if (e == text || *e != '\0' || v < 1 || v > 1000000) return fail(t, "TSDR_SPECTRUM: expected <nfft>, an integer", TSDR_INVALID_PARAMETER_VALUE);
+	if (!file || !file[0]) return fail(t, "TSDR_SPECTRUM: needs TSDR_SPECTRUM_FILE=<path> for the spectrum", TSDR_INVALID_PARAMETER_VALUE);
+	if (tsdrgpu_spectrum_check(t->samplerate_real, (int) v) != TSDRGPU_OK) return fail(t, tsdrgpu_last_error(NULL), TSDR_INVALID_PARAMETER_VALUE);
+	t->sp_nfft = (int) v; t->sp_file = file;
+	return TSDR_OK;
+}
+
+/* the spectrum as CSV, frequency ascending, density in dB per Hz */
+static void write_spectrum(tsdr_lib_t *t, tsdrgpu_pipeline_t *p) {
+	static double psd[16384];
+	int n = 0; uint64_t segs = 0;
+	if (tsdrgpu_pipeline_spectrum(p, psd, 16384, &n, &segs) != TSDRGPU_OK) return;
+	FILE *f = fopen(t->sp_file, "w");
+	if (!f) return;
+	fprintf(f, "frequency_hz,psd_db_per_hz\n");
+	for (int i = 0; i < n; i++)
+		fprintf(f, "%.3f,%.6f\n", ((double) i - n / 2) * (double) t->samplerate_real / n, psd[i] > 0.0 ? 10.0 * log10(psd[i]) : -400.0);
+	fclose(f);
 }
 
 /* the scan's table as CSV, one row per channel, highest frame_score first (ties: lower channel first) */
@@ -408,7 +470,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	tsdr_reset(t);
 	t->nativerunning = 1; t->running = 1; t->gpu_failed = 0;
 	int status, pluginsfault = 0;
-	t->tuner_d = 1; t->tn_bw = 0.0; t->sc_k = 0;
+	t->tuner_d = 1; t->tn_bw = 0.0; t->sc_k = 0; t->nt_n = 0; t->sp_nfft = 0;
 	if ((status = tsdr_getsamplerate(t)) != TSDR_OK) goto end;
 	{
 		const char *tuner = getenv("TSDR_TUNER");
@@ -418,6 +480,10 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 		}
 		const char *scan = getenv("TSDR_SCAN");
 		if (scan && scan[0] && (status = parse_scan(t, scan, getenv("TSDR_SCAN_FILE"))) != TSDR_OK) goto end;
+		const char *notch = getenv("TSDR_NOTCH");
+		if (notch && notch[0] && (status = parse_notch(t, notch, getenv("TSDR_NOTCH_TAPS"))) != TSDR_OK) goto end;
+		const char *spec = getenv("TSDR_SPECTRUM");
+		if (spec && spec[0] && (status = parse_spectrum(t, spec, getenv("TSDR_SPECTRUM_FILE"))) != TSDR_OK) goto end;
 	}
 	if (t->width <= 0 || t->height <= 0 || (long long) t->width * t->height > MAX_PIXELS) {
 		status = fail(t, "The supplied height and the width are invalid!", TSDR_WRONG_VIDEOPARAMS);
@@ -474,6 +540,12 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 			tsdrgpu_pipeline_destroy(np);
 			goto end;
 		}
+		if ((t->nt_n > 0 && tsdrgpu_pipeline_set_notches(np, t->nt_n, t->nt_centers, t->nt_widths, t->nt_taps) != TSDRGPU_OK) ||
+		    (t->sp_nfft > 0 && tsdrgpu_pipeline_set_spectrum(np, t->sp_nfft) != TSDRGPU_OK)) {
+			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_INVALID_PARAMETER_VALUE);
+			tsdrgpu_pipeline_destroy(np);
+			goto end;
+		}
 		if (ndev > 1 && tsdrgpu_pipeline_set_superb_devices(np, devlist, ndev) != TSDRGPU_OK) {
 			status = fail(t, tsdrgpu_last_error(t->gpu), TSDR_CANNOT_OPEN_DEVICE);
 			tsdrgpu_pipeline_destroy(np);
@@ -505,6 +577,7 @@ int tsdr_readasync(tsdr_lib_t *t, tsdr_readasync_function cb, void *ctx) {
 	}
 	tsdrgpu_pipeline_flush(t->pipe);
 	if (t->sc_k > 0) write_scan(t, t->pipe);
+	if (t->sp_nfft > 0) write_spectrum(t, t->pipe);
 	{
 		pthread_rwlock_wrlock(&t->pipe_lock);        /* no setter is inside the object any more, none can enter */
 		tsdrgpu_pipeline_t *p = t->pipe;

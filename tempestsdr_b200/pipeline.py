@@ -26,6 +26,7 @@ class Pipeline:
                  on_frame: Optional[Callable] = None, on_value: Optional[Callable] = None, on_plot: Optional[Callable] = None,
                  on_retune: Optional[Callable] = None):
         self._lib = N.lib()
+        self._samplerate = int(samplerate)
         ctx = C.c_void_p()
         N.check(self._lib.tsdrgpu_create(C.byref(ctx), device))
         self._ctx = ctx
@@ -133,8 +134,33 @@ class Pipeline:
         N.check(self._lib.tsdrgpu_pipeline_scan_results(self._h, recs, 256, C.byref(n)), self._ctx)
         return scan_table(recs, n.value)
 
+    def set_notches(self, centers, widths, ntaps: int = 0) -> None:
+        """Remove the stopbands (centers[j], widths[j]) in Hz from every block before anything else reads it (empty lists switch
+        the notch off).  Takes effect at the next process() call, which starts the stream over behind the notch."""
+        c = np.ascontiguousarray(centers, dtype=np.float64)
+        w = np.ascontiguousarray(widths, dtype=np.float64)
+        assert c.shape == w.shape and c.ndim == 1, "one width per center"
+        N.check(self._lib.tsdrgpu_pipeline_set_notches(self._h, c.size, c.ctypes.data_as(C.c_void_p), w.ctypes.data_as(C.c_void_p),
+                                                       int(ntaps)), self._ctx)
+
+    def set_spectrum(self, nfft: int) -> None:
+        """Accumulate the power spectrum of the blocks as received, with nfft bins (0 switches it off).  Takes effect, reset, at the
+        next process() call; the pixel path is not affected."""
+        N.check(self._lib.tsdrgpu_pipeline_set_spectrum(self._h, int(nfft)), self._ctx)
+
+    def spectrum(self):
+        """(frequencies in Hz, density per Hz, segments averaged), fft-shifted; empty arrays while no spectrum runs."""
+        from .api import spectrum_freqs
+        nfft = 16384
+        psd = np.zeros(nfft, np.float64)
+        n, segs = C.c_int(0), C.c_uint64(0)
+        N.check(self._lib.tsdrgpu_pipeline_spectrum(self._h, psd.ctypes.data_as(C.c_void_p), nfft, C.byref(n), C.byref(segs)), self._ctx)
+        fs = self._samplerate
+        return spectrum_freqs(fs, n.value), psd[: n.value].copy(), segs.value
+
     def set_samplerate(self, samplerate: int) -> None:
         N.check(self._lib.tsdrgpu_pipeline_set_samplerate(self._h, int(samplerate)), self._ctx)
+        self._samplerate = int(samplerate)
 
     def set_superb_devices(self, devices) -> None:
         """Superbandwidth mode with one hop per GPU: devices[0] is this pipeline's device, len(devices) in {2, 4, 8} = hops."""
